@@ -187,6 +187,15 @@ def run_ours(args):
     e.record()
     barrier()
     dev_ms = max_over_ranks(s.elapsed_time(e))
+    if args.dump_outputs:
+        # what the timed decode hands its caller (the greedy tokens) and the full-vocabulary logits row of its last step, read
+        # before the decodes below overwrite the logits buffer
+        logits = eng.logits[0] if world == 1 else comm.all_gather_cat(eng.logits[0], dim=-1)
+        if rank == 0:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "tokens.npy"), np.asarray(toks, dtype=np.float64))
+            np.save(os.path.join(args.dump_outputs, "logits.npy"), logits.float().cpu().numpy())
     # long-context decode: the same step at position 2048 (the KV rows below it hold whatever the cache was initialised with —
     # only the attention cost over 2048 positions is of interest)
     extra = {}
@@ -274,15 +283,16 @@ def run_ours(args):
 
 # ------------------------------------------------------------------------------------------------------------
 def ref_binary():
-    src = os.path.join(ROOT, "baseline", "_ref", "distributed-llama")
+    """The reference tree that oracle/build_reference.sh put under oracle/_ref/, copied to the cache directory and built there
+    (the repository may be read-only)."""
+    tree = os.path.join(ROOT, "oracle", "_ref", "distributed-llama")
+    if not os.path.isdir(tree):
+        return None, "reference sources not present under oracle/_ref (oracle/build_reference.sh)"
+    src = os.path.join(CACHE_DIR, "reference")
     exe = os.path.join(src, "dllama")
     if not os.path.isdir(src):
-        if os.path.isdir("/root/reference"):
-            os.makedirs(os.path.dirname(src), exist_ok=True)
-            shutil.copytree("/root/reference", src)
-            subprocess.run(["chmod", "-R", "u+w", src])
-        else:
-            return None, "reference sources not present under baseline/_ref"
+        shutil.copytree(tree, src)
+        subprocess.run(["chmod", "-R", "u+w", src])
     # always (re)build on the box we run on: the reference Makefile uses -march=native
     stamp = os.path.join(src, ".built_on")
     host_id = open("/proc/cpuinfo").read().split("model name")[1].split("\n")[0] if os.path.exists("/proc/cpuinfo") else "?"
@@ -360,7 +370,7 @@ def _run_reference_once(exe, args, model_path, tok_path, n, threads, steps, warm
 
 
 def run_reference(args):
-    """Reference arm: the UNMODIFIED reference tree (baseline/_ref/distributed-llama), built with its own Makefile, driven through
+    """Reference arm: the UNMODIFIED reference tree (oracle/_ref/distributed-llama), built with its own Makefile, driven through
     its own CLI. The only thing chosen here is how it is launched: `--nthreads` is swept over the power-of-two counts that fit the
     physical cores available to each of the n processes (short probe runs), processes are pinned to disjoint CPU sets, and the
     best configuration is then timed on the full step count."""
@@ -440,6 +450,7 @@ def main():
     ap.add_argument("--max-seq-len", type=int, default=4096)
     ap.add_argument("--ref-timeout", type=int, default=1500)
     ap.add_argument("--decode-path", default="mega", choices=["multi", "mega"], help="multi-kernel PDL chain or persistent megakernel")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed decode's tokens and last-step logits as DIR/*.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -78,8 +78,9 @@ class RootInference:
         self.header = sess.header
         self.eval_ms = 0.0
         self._ctl = torch.zeros(4, dtype=torch.int64, device=sess.device) if (comm is not None and chan is None) else None
-        self._pin_out = torch.zeros(1, dtype=torch.int32).pin_memory() if torch.cuda.is_available() else None
-        self._pin_in = torch.zeros(2, dtype=torch.int32).pin_memory() if torch.cuda.is_available() else None
+        on_gpu = sess.device.type == "cuda"
+        self._pin_out = torch.zeros(1, dtype=torch.int32).pin_memory() if on_gpu else None
+        self._pin_in = torch.zeros(2, dtype=torch.int32).pin_memory() if on_gpu else None
 
     def _send(self, op: int, pos: int, tokens: Sequence[int]):
         if self.comm is None:
@@ -106,7 +107,7 @@ class RootInference:
 
     def forward_greedy(self, token: int, pos: int) -> int:
         self._send(OP_STEP_GREEDY, pos, [token])
-        if self._pin_in is None:          # no CUDA device (CPU-side protocol tests)
+        if self._pin_in is None:          # session on the CPU (protocol tests)
             self.eng._set_inputs([token], pos)
             self.eng.run_decode_step()
             return int(self.eng.tokens[0])
