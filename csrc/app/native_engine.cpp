@@ -59,12 +59,9 @@ struct NativeEngine::Impl {
     struct Layer {
         Q40Dev qkv, wo, w13, w2;
         float *norm0 = nullptr, *norm1 = nullptr, *qNorm = nullptr, *kNorm = nullptr, *moeGate = nullptr;
-        void *kCache = nullptr, *vCache = nullptr;
     };
     std::vector<Layer> layers;
-    // activations / state
-    int32_t *tokens = nullptr, *pos = nullptr, *history = nullptr, *pTokens = nullptr, *pPos = nullptr;
-    float *logits = nullptr;
+    EngineBuffers buf{};   // engine-owned inputs / outputs
     std::vector<float> hostLogits;
     std::map<std::tuple<std::string, uint32_t, uint32_t>, const TensorEntry *> index;
     const TensorEntry &entry(const std::string &name, uint32_t layer = 0, uint32_t expert = 0) const {
@@ -97,8 +94,6 @@ NativeEngine::NativeEngine(const std::string &modelPath, uint32_t maxSeqLen, int
         cudaCheck(cudaSetDevice(device), "cudaSetDevice");
         cudaCheck(cudaStreamCreateWithFlags(&impl_->stream, cudaStreamNonBlocking), "cudaStreamCreate");
         for (const TensorEntry &t : dir_) impl_->index[std::make_tuple(t.name, t.layer, t.expert)] = &t;
-        int sms = 0;
-        cudaCheck(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device), "cudaDeviceGetAttribute");
         const uint32_t hd = h_.headDim, dim = h_.dim, vocab = h_.vocabSize, N = nRanks_;
         // tensor-parallel placement (same rules as distributed_llama_b200/models/loader.py; reference slicers src/nn/nn-core.cpp:223-322):
         // more ranks than KV heads -> nRanks / nKvHeads ranks share one KV head, each with its own query heads of that group
@@ -118,82 +113,51 @@ NativeEngine::NativeEngine(const std::string &modelPath, uint32_t maxSeqLen, int
         if (N > 1 && (qDim % 128 || ff % 128))
             throw std::runtime_error("per-GPU slices of WO / W2 must be multiples of 128 columns (use fewer GPUs)");
         qkvDim_ = qDim + 2 * kvDim;
-        const bool moe = h_.nExperts > 0;
-        maxBatch_ = moe ? 1 : 8;
-        nSplits_ = (uint32_t)std::max(1, std::min(32, (2 * sms) / (int)std::max(1u, headsL_)));
 
         Mapping file(modelPath);
         uploadWeights(file.data);
 
-        // ---- activation buffers (sizes as in distributed_llama_b200/runtime/engine.py) ----
         Impl &I = *impl_;
-        const uint32_t mb = maxBatch_, mp = maxPrefill_, kAct = std::max(1u, h_.nActiveExperts);
-        I.tokens = (int32_t *)dev(mb * 4); I.pos = (int32_t *)dev(mb * 4);
-        float *x = (float *)dev((size_t)mb * dim * 4), *qkv = (float *)dev((size_t)mb * qkvDim_ * 4), *z = (float *)dev((size_t)mb * qDim * 4);
-        float *hbuf = (float *)dev((size_t)std::max(mb, kAct) * ff * 4);
-        I.logits = (float *)dev((size_t)mb * vocabL_ * 4);
         I.hostLogits.resize(vocab);
-        I.history = (int32_t *)dev((size_t)(seqLen_ + 1) * 4);
-        I.pTokens = (int32_t *)dev(mp * 4); I.pPos = (int32_t *)dev(mp * 4);
-        GlobalPtrs g{};
-        g.embedding = I.embedding; g.finalNorm = I.finalNorm; g.wclsQs = I.wcls.qs; g.wclsSc = I.wcls.scales; g.rope = I.rope;
-        g.vocabFull = vocab; g.tokens = I.tokens; g.pos = I.pos; g.x = x; g.qkv = qkv; g.z = z; g.h = hbuf; g.logits = I.logits;
-        g.attnPartial = (float *)dev((size_t)mb * headsL_ * nSplits_ * (hd + 2) * 4);
-        g.attnCounters = (unsigned int *)dev((size_t)mb * headsL_ * 4);
-        g.history = I.history;
-        g.expertIdx = (int *)dev((size_t)mb * kAct * 4); g.expertWeight = (float *)dev((size_t)mb * kAct * 4);
-        g.routerLogits = (float *)dev((size_t)mb * std::max(1u, h_.nExperts) * 4); g.routerCounter = (unsigned int *)dev(mb * 4);
-        g.moeScratch = (float *)dev((size_t)kAct * dim * 4); g.moeCounters = (unsigned int *)dev(256 * 4);
-        g.maxPrefill = mp; g.pTokens = I.pTokens; g.pPos = I.pPos;
-        g.px = (float *)dev((size_t)mp * dim * 4); g.pqkv = (float *)dev((size_t)mp * std::max(qkvDim_, dim) * 4);   // also the [T][dim] partial product of the tensor-parallel WO / W2 GEMMs
-        g.pxn = dev((size_t)mp * dim * 2); g.pzb = dev((size_t)mp * qDim * 2); g.phb = dev((size_t)mp * ff * 2);
-        g.pAttnPartial = (float *)dev((size_t)mp * headsL_ * (hd + 2) * 4); g.pAttnCounters = (unsigned int *)dev((size_t)mp * headsL_ * 4);
-        g.argVal = (float *)dev(256 * 4); g.argIdx = (int *)dev(256 * 4); g.argCounter = (unsigned int *)dev(16);
-
         EngineConfig cfg{};
         cfg.dim = dim; cfg.nLayers = h_.nLayers; cfg.nHeads = headsL_; cfg.nKvHeads = kvHeadsL_; cfg.headDim = hd; cfg.ffDim = ff;
-        cfg.vocab = vocabL_; cfg.seqLen = seqLen_; cfg.nExperts = h_.nExperts; cfg.nActiveExperts = h_.nActiveExperts; cfg.maxBatch = mb;
-        cfg.nSplits = nSplits_; cfg.rank = rank_; cfg.nRanks = N; cfg.numSms = (uint32_t)sms; cfg.eps = h_.normEpsilon; cfg.usePdl = 1;
+        cfg.vocab = vocabL_; cfg.seqLen = seqLen_; cfg.nExperts = h_.nExperts; cfg.nActiveExperts = h_.nActiveExperts; cfg.maxBatch = maxBatch_;
+        cfg.rank = rank_; cfg.nRanks = N; cfg.eps = h_.normEpsilon; cfg.usePdl = 1;
         cfg.moeFirstExpert = 0; cfg.moeNumLocal = h_.nExperts; cfg.wType = 0;
         cfg.hiddenAct = h_.hiddenAct == ACT_GELU ? 1u : 0u;
+        cfg.vocabFull = vocab; cfg.maxPrefill = maxPrefill_;
         I.engine = dl_engine_create(&cfg);
         if (!I.engine) throw std::runtime_error("dl_engine_create failed");
+        engCheck(dl_engine_get_config(I.engine, &cfg), "dl_engine_get_config");
+        maxBatch_ = cfg.maxBatch; maxPrefill_ = cfg.maxPrefill;
+        engCheck(dl_engine_buffers(I.engine, &I.buf), "dl_engine_buffers");
         for (uint32_t l = 0; l < h_.nLayers; l++) {
             const Impl::Layer &L = I.layers[l];
             LayerPtrs lp{};
             lp.qkvQs = L.qkv.qs; lp.qkvSc = L.qkv.scales; lp.woQs = L.wo.qs; lp.woSc = L.wo.scales;
             lp.w13Qs = L.w13.qs; lp.w13Sc = L.w13.scales; lp.w2Qs = L.w2.qs; lp.w2Sc = L.w2.scales;
             lp.norm0 = L.norm0; lp.norm1 = L.norm1; lp.qNorm = L.qNorm; lp.kNorm = L.kNorm; lp.moeGate = L.moeGate;
-            lp.kCache = L.kCache; lp.vCache = L.vCache;
             engCheck(dl_engine_set_layer(I.engine, l, &lp), "dl_engine_set_layer");
         }
+        GlobalPtrs g{};
+        g.embedding = I.embedding; g.finalNorm = I.finalNorm; g.wclsQs = I.wcls.qs; g.wclsSc = I.wcls.scales; g.rope = I.rope;
         engCheck(dl_engine_set_globals(I.engine, &g), "dl_engine_set_globals");
         if (N > 1) {
-            // symmetric peer-memory arena, same layout as distributed_llama_b200/parallel/comm.py:arena_layout
-            auto align = [](uint64_t x) { return (x + 255) / 256 * 256; };
-            const uint32_t maxCtas = 256;
-            CommPtrs cp{};
-            uint64_t off = 0;
-            cp.slotsOff = off; off = align(off + 2ull * N * mb * dim * 8);            // LL words of the decode all-reduce
-            cp.flagsOff = off; off = align(off + 2ull * N * maxCtas * 4);             // logits-gather arrival counters
-            cp.candValOff = off; off = align(off + 8 * 8);                            // cross-rank arg-max candidates
-            cp.gatherOff = off; off = align(off + (uint64_t)mb * vocab * 4);          // gathered logits (device sampler)
-            cp.prefillSlotsOff = off; off = align(off + 2ull * N * mp * dim * 8);     // LL words of the prefill all-reduce
-            I.vmm = dl_vmm_create(rank_, N, off, commTag.c_str(), 1);
+            const size_t bytes = dl_engine_arena_bytes(&cfg);   // symmetric peer-memory arena
+            I.vmm = dl_vmm_create(rank_, N, bytes, commTag.c_str(), 1);
             if (!I.vmm) throw std::runtime_error("cannot create the peer-memory arena (CUDA VMM with POSIX file-descriptor handles is required)");
             if (hostBarrier) hostBarrier();      // every rank has bound its bootstrap socket
             engCheck(dl_vmm_connect(I.vmm), "dl_vmm_connect");
-            cudaCheck(cudaMemsetAsync(dl_vmm_ptr(I.vmm, rank_), 0, off, I.stream), "cudaMemset(arena)");
+            cudaCheck(cudaMemsetAsync(dl_vmm_ptr(I.vmm, rank_), 0, bytes, I.stream), "cudaMemset(arena)");
             cudaCheck(cudaStreamSynchronize(I.stream), "cudaMemset(arena)");
             engCheck(dl_vmm_barrier(I.vmm, 3), "dl_vmm_barrier");   // nobody pushes into an arena that is still being cleared
-            cp.nRanks = N; cp.rank = rank_; cp.maxCtas = maxCtas; cp.slotStride = mb * dim;
+            CommPtrs cp{};
             for (uint32_t r = 0; r < N; r++) cp.arena[r] = dl_vmm_ptr(I.vmm, r);
             cp.mcArena = dl_vmm_mc_ptr(I.vmm);
             multicast_ = cp.mcArena != nullptr;
-            cp.prefillSlotStride = mp * dim;
             engCheck(dl_engine_set_comm(I.engine, &cp), "dl_engine_set_comm");
         }
-        if (!moe) {
+        if (h_.nExperts == 0) {
             engCheck(dl_engine_enable_mega(I.engine, 1), "dl_engine_enable_mega");   // falls back per call if the shape is unsupported
             mega_ = true;
         }
@@ -314,8 +278,6 @@ void NativeEngine::uploadWeights(const uint8_t *file) {
             L.kNorm = f32Tensor(I.entry("block_norm_k", l), neox ? &perm : nullptr);
         }
         if (h_.nExperts > 0) L.moeGate = f32Tensor(I.entry("block_moe_gate", l));
-        L.kCache = dev((size_t)kvHeadsL_ * seqLen_ * hd * 2);
-        L.vCache = dev((size_t)kvHeadsL_ * seqLen_ * hd * 2);
     }
     cudaCheck(cudaStreamSynchronize(st), "weight upload");
     cudaFree(staging);
@@ -326,8 +288,8 @@ void NativeEngine::setInputs(const int32_t *tokens, uint32_t n, uint32_t pos, bo
     for (uint32_t i = 0; i < n; i++) p[i] = (int32_t)(pos + i);
     Impl &I = *impl_;
     // pageable sources: the copies are staged before the call returns, so the vectors may die right away
-    cudaCheck(cudaMemcpyAsync(prefillBuffers ? I.pTokens : I.tokens, tokens, n * 4, cudaMemcpyHostToDevice, I.stream), "cudaMemcpy(tokens)");
-    cudaCheck(cudaMemcpyAsync(prefillBuffers ? I.pPos : I.pos, p.data(), n * 4, cudaMemcpyHostToDevice, I.stream), "cudaMemcpy(pos)");
+    cudaCheck(cudaMemcpyAsync(prefillBuffers ? I.buf.pTokens : I.buf.tokens, tokens, n * 4, cudaMemcpyHostToDevice, I.stream), "cudaMemcpy(tokens)");
+    cudaCheck(cudaMemcpyAsync(prefillBuffers ? I.buf.pPos : I.buf.pos, p.data(), n * 4, cudaMemcpyHostToDevice, I.stream), "cudaMemcpy(pos)");
 }
 
 void NativeEngine::forward(uint32_t n, int logitsMode, bool greedyAdvance) {
@@ -361,7 +323,7 @@ const float *NativeEngine::step(int32_t token, uint32_t pos) {
     setInputs(&token, 1, pos, false);
     forward(1, 1, false);
     Impl &I = *impl_;
-    cudaCheck(cudaMemcpyAsync(I.hostLogits.data(), I.logits, (size_t)h_.vocabSize * 4, cudaMemcpyDeviceToHost, I.stream), "cudaMemcpy(logits)");
+    cudaCheck(cudaMemcpyAsync(I.hostLogits.data(), I.buf.logits, (size_t)h_.vocabSize * 4, cudaMemcpyDeviceToHost, I.stream), "cudaMemcpy(logits)");
     cudaCheck(cudaStreamSynchronize(I.stream), "step");
     return I.hostLogits.data();
 }
@@ -380,7 +342,7 @@ std::vector<int32_t> NativeEngine::decodeGreedy(int32_t firstToken, uint32_t pos
     }
     engCheck(dl_engine_decode_graph(I.engine, (int)nSteps, I.stream), "dl_engine_decode_graph");
     std::vector<int32_t> out(nSteps);
-    cudaCheck(cudaMemcpyAsync(out.data(), I.history + pos + 1, (size_t)nSteps * 4, cudaMemcpyDeviceToHost, I.stream), "cudaMemcpy(history)");
+    cudaCheck(cudaMemcpyAsync(out.data(), I.buf.history + pos + 1, (size_t)nSteps * 4, cudaMemcpyDeviceToHost, I.stream), "cudaMemcpy(history)");
     cudaCheck(cudaStreamSynchronize(I.stream), "decode");
     return out;
 }
@@ -398,7 +360,7 @@ int32_t NativeEngine::stepGreedy(int32_t token, uint32_t pos) {
     }
     engCheck(dl_engine_decode_graph(I.engine, 1, I.stream), "dl_engine_decode_graph");
     int32_t next = 0;   // the arg-max kernel leaves the sampled token in tokens[0] (and advances pos[0]) on the device
-    cudaCheck(cudaMemcpyAsync(&next, I.tokens, 4, cudaMemcpyDeviceToHost, I.stream), "cudaMemcpy(token)");
+    cudaCheck(cudaMemcpyAsync(&next, I.buf.tokens, 4, cudaMemcpyDeviceToHost, I.stream), "cudaMemcpy(token)");
     cudaCheck(cudaStreamSynchronize(I.stream), "stepGreedy");
     if (nRanks_ > 1 && dl_engine_aborted(I.engine)) throw std::runtime_error("device-side wait timed out: a tensor-parallel peer stopped responding");
     return next;
@@ -413,7 +375,7 @@ int32_t NativeEngine::stepSampled(int32_t token, uint32_t pos, float temperature
     forward(1, 1, false);
     engCheck(dl_engine_sample(I.engine, temperature, topp, I.stream), "dl_engine_sample");
     int32_t next = 0;   // the sampler leaves the drawn token in tokens[0]
-    cudaCheck(cudaMemcpyAsync(&next, I.tokens, 4, cudaMemcpyDeviceToHost, I.stream), "cudaMemcpy(token)");
+    cudaCheck(cudaMemcpyAsync(&next, I.buf.tokens, 4, cudaMemcpyDeviceToHost, I.stream), "cudaMemcpy(token)");
     cudaCheck(cudaStreamSynchronize(I.stream), "stepSampled");
     if (dl_engine_aborted(I.engine)) throw std::runtime_error("device-side wait timed out: a tensor-parallel peer stopped responding");
     return next;

@@ -1,4 +1,4 @@
-// Python-free runtime of one GPU: maps a `.m` file, uploads + re-tiles the q40 weights, owns the device buffers and drives the
+// Python-free runtime of one GPU: maps a `.m` file, uploads + re-tiles the q40 weights and drives the
 // engine in _cuda.so (persistent decode kernel, tcgen05 prefill, CUDA-graph greedy loop).
 //
 // Role in the reference: loadLlmNetWeight + NnExecutor/NnCpuDevice set-up + RootLlmInference (src/llm.cpp:614-669,
@@ -63,7 +63,7 @@ public:
 
 private:
     struct Impl;
-    void *dev(size_t bytes);            // zero-initialised device allocation owned by the engine
+    void *dev(size_t bytes);            // zero-initialised device allocation for weights, owned by the engine
     void release();
     void uploadWeights(const uint8_t *file);
     void setInputs(const int32_t *tokens, uint32_t n, uint32_t pos, bool prefillBuffers);
@@ -71,7 +71,7 @@ private:
 
     ModelHeader h_;
     std::vector<TensorEntry> dir_;
-    uint32_t seqLen_ = 0, maxBatch_ = 8, maxPrefill_ = 192, nSplits_ = 1, qkvDim_ = 0;
+    uint32_t seqLen_ = 0, maxBatch_ = 8, maxPrefill_ = 192, qkvDim_ = 0;
     uint32_t rank_ = 0, nRanks_ = 1, kvRank_ = 0, kvSlices_ = 1;          // tensor-parallel placement of this process
     uint32_t headsL_ = 0, kvHeadsL_ = 0, ffL_ = 0, vocabL_ = 0;          // per-rank slice sizes
     bool mega_ = false, graphReady_ = false, multicast_ = false;

@@ -6,6 +6,7 @@
 // programmatic dependent launch, and the single-token step is captured once into a CUDA graph whose inputs
 // (token id, position) live in device memory so the graph replays without host round trips:
 // the sampling kernel writes the next token and advances the position on the device.
+#include <algorithm>
 #include <cstdlib>
 #include <cstring>
 #include <vector>
@@ -19,11 +20,40 @@ uint32_t gHiddenAct = 0;
 
 static_assert(kApiMaxRanks == kMaxRanks, "engine_api.h and kernels.h disagree on the rank limit");
 
+struct Buffers {   // working memory of the kernels, allocated and zeroed by dl_engine_create
+    int *tokens, *pos;           // [maxBatch]
+    float *x, *qkv, *z, *h, *logits;   // [maxBatch][dim | qkvDim | qDim | ff | vocab] (h: max(maxBatch, nActive) rows)
+    float *attnPartial;          // [maxBatch][nHeads][nSplits][hd+2]
+    unsigned int *attnCounters;  // [maxBatch][nHeads]
+    int *history;                // [seqLen + 1] generated token per position (device-side log)
+    // MoE scratch
+    int *expertIdx;              // [maxBatch][nActive]
+    float *expertWeight;         // [maxBatch][nActive]
+    float *routerLogits;         // [maxBatch][nExperts]
+    unsigned int *routerCounter; // [maxBatch]
+    float *moeScratch;           // [nActive][dim]
+    unsigned int *moeCounters;   // [256]
+    // prefill (tensor-core GEMM path) buffers, maxPrefill tokens
+    int *pTokens, *pPos;         // [maxPrefill]
+    float *px, *pqkv;            // [maxPrefill][dim | max(qkvDim, dim)] f32; pqkv also takes the [T][dim] partial of the TP WO / W2 GEMMs
+    void *pxn, *pzb, *phb;       // bf16 [maxPrefill][dim | qDim | ff]
+    float *pAttnPartial;         // [maxPrefill][nHeads][hd+2]
+    unsigned int *pAttnCounters; // [maxPrefill][nHeads]
+    // fused arg-max scratch
+    float *argVal;               // [256]
+    int *argIdx;                 // [256]
+    unsigned int *argCounter;    // [4]
+};
+
 struct Engine {
     EngineConfig cfg{};
     CommPtrs comm{};
+    bool tp = false;             // dl_engine_set_comm was called: all-reduces run inside the kernels over the peer arena
     std::vector<LayerPtrs> layers;
     GlobalPtrs g{};
+    Buffers b{};
+    std::vector<void *> kCache, vCache;   // per layer, bf16 [nKvHeads][seqLen][hd]
+    std::vector<void *> owned;            // device allocations freed by dl_engine_destroy
     cudaGraphExec_t decodeGraph = nullptr;
     cudaStream_t captureStream = nullptr;
     int lastError = 0;
@@ -67,14 +97,41 @@ static EmbTable embTable(const Engine &e) {
     return t;
 }
 
+constexpr uint32_t kArenaMaxCtas = 256;   // logits-gather arrival counters per rank and parity
+
+// The limits both front ends rely on: the MoE kernels route one token per launch, enginePrefill takes at most 256 tokens.
+static EngineConfig applyLimits(EngineConfig c) {
+    if (c.nExperts > 0) c.maxBatch = 1;
+    if (c.maxPrefill > 256) c.maxPrefill = 256;
+    return c;
+}
+
+struct ArenaLayout {   // byte offsets into every rank's peer arena, 256-byte aligned
+    uint64_t slotsOff, flagsOff, candValOff, gatherOff, prefillSlotsOff, bytes;
+};
+
+static ArenaLayout arenaLayout(const EngineConfig &c) {
+    auto align = [](uint64_t x) { return (x + 255) / 256 * 256; };
+    ArenaLayout a{};
+    uint64_t off = 0;
+    a.slotsOff = off; off = align(off + 2ull * c.nRanks * c.maxBatch * c.dim * 8);            // LL words (f32 payload, flag) of the decode all-reduce
+    a.flagsOff = off; off = align(off + 2ull * c.nRanks * kArenaMaxCtas * 4);                // logits-gather arrival counters (sampler.cu)
+    a.candValOff = off; off = align(off + kMaxRanks * 8);                                    // arg-max candidates, one LL word per rank
+    a.gatherOff = off; off = align(off + (uint64_t)c.maxBatch * c.vocabFull * 4);            // gathered logits (device sampler)
+    a.prefillSlotsOff = off; off = align(off + 2ull * c.nRanks * c.maxPrefill * c.dim * 8);  // LL words of the prefill all-reduce
+    a.bytes = off;
+    return a;
+}
+
 static void fillAr(const Engine &e, ArArgs &ar, uint32_t parity) {
-    const CommPtrs &c = e.comm;
-    ar.nRanks = c.nRanks; ar.rank = c.rank; ar.parity = parity; ar.maxCtas = c.maxCtas; ar.slotStride = c.slotStride; ar.dim = e.cfg.dim;
-    ar.slotsMc = c.mcArena ? (uint64_t *)((uint8_t *)c.mcArena + c.slotsOff) : nullptr;
+    const EngineConfig &c = e.cfg;
+    const ArenaLayout L = arenaLayout(c);
+    ar.nRanks = c.nRanks; ar.rank = c.rank; ar.parity = parity; ar.maxCtas = kArenaMaxCtas; ar.slotStride = c.maxBatch * c.dim; ar.dim = c.dim;
+    ar.slotsMc = e.comm.mcArena ? (uint64_t *)((uint8_t *)e.comm.mcArena + L.slotsOff) : nullptr;
     for (uint32_t r = 0; r < c.nRanks && r < (uint32_t)kMaxRanks; r++) {
-        uint8_t *base = (uint8_t *)c.arena[r];
-        ar.slots[r] = (uint64_t *)(base + c.slotsOff);
-        ar.cand[r] = (uint64_t *)(base + c.candValOff);
+        uint8_t *base = (uint8_t *)e.comm.arena[r];
+        ar.slots[r] = (uint64_t *)(base + L.slotsOff);
+        ar.cand[r] = (uint64_t *)(base + L.candValOff);
     }
 }
 
@@ -98,24 +155,24 @@ static int runMoe(Engine &e, const LayerPtrs &L, float *out, bool fusedAr, uint6
     const EngineConfig &c = e.cfg;
     if (c.wType != 0) return -34;   // expert-indexed kernels exist for q40 matrices only
     RouterArgs ro{};
-    ro.x = e.g.x; ro.normW = L.norm1; ro.gate = L.moeGate; ro.eps = c.eps; ro.dim = c.dim; ro.nExperts = c.nExperts;
-    ro.k = c.nActiveExperts; ro.logits = e.g.routerLogits; ro.counter = e.g.routerCounter; ro.expertIdx = e.g.expertIdx;
-    ro.expertWeight = e.g.expertWeight;
+    ro.x = e.b.x; ro.normW = L.norm1; ro.gate = L.moeGate; ro.eps = c.eps; ro.dim = c.dim; ro.nExperts = c.nExperts;
+    ro.k = c.nActiveExperts; ro.logits = e.b.routerLogits; ro.counter = e.b.routerCounter; ro.expertIdx = e.b.expertIdx;
+    ro.expertWeight = e.b.expertWeight;
     DL_TRY(launchMoeRouter(ro, 1, stream, pdl));
     const uint32_t perSlot = c.numSms / c.nActiveExperts > 0 ? c.numSms / c.nActiveExperts : 1;
     GemvArgs a{};
     a.qs = (const uint32_t *)L.w13Qs; a.scales = (const __half *)L.w13Sc; a.d = 2 * c.ffDim; a.n = c.dim;
-    a.in = e.g.x; a.inStride = c.dim; a.normW = L.norm1; a.eps = c.eps; a.out = e.g.h; a.outStride = c.ffDim; a.trace = trace13;
-    a.moeCtasPerSlot = perSlot; a.kActive = c.nActiveExperts; a.expertIdx = e.g.expertIdx; a.outSlotStride = c.ffDim;
+    a.in = e.b.x; a.inStride = c.dim; a.normW = L.norm1; a.eps = c.eps; a.out = e.b.h; a.outStride = c.ffDim; a.trace = trace13;
+    a.moeCtasPerSlot = perSlot; a.kActive = c.nActiveExperts; a.expertIdx = e.b.expertIdx; a.outSlotStride = c.ffDim;
     a.expertQsStride = (uint64_t)2 * c.ffDim * (c.dim / 8); a.expertScaleStride = (uint64_t)2 * c.ffDim * (c.dim / 32);
     a.moeFirstExpert = c.moeFirstExpert; a.moeNumLocal = c.moeNumLocal;
     { const int r = gemvQ40Tma(PRO_RMSNORM_, EPI_SWIGLU_, 1, a, c.numSms, stream, pdl); if (r != 0) return r == 1 ? -31 : r; }
     a = GemvArgs{};
     a.qs = (const uint32_t *)L.w2Qs; a.scales = (const __half *)L.w2Sc; a.d = c.dim; a.n = c.ffDim;
-    a.in = e.g.h; a.inStride = c.ffDim; a.inSlotStride = c.ffDim; a.out = out; a.outStride = c.dim; a.trace = trace2;
-    a.moeCtasPerSlot = perSlot; a.kActive = c.nActiveExperts; a.expertIdx = e.g.expertIdx; a.expertWeight = e.g.expertWeight;
+    a.in = e.b.h; a.inStride = c.ffDim; a.inSlotStride = c.ffDim; a.out = out; a.outStride = c.dim; a.trace = trace2;
+    a.moeCtasPerSlot = perSlot; a.kActive = c.nActiveExperts; a.expertIdx = e.b.expertIdx; a.expertWeight = e.b.expertWeight;
     a.expertQsStride = (uint64_t)c.dim * (c.ffDim / 8); a.expertScaleStride = (uint64_t)c.dim * (c.ffDim / 32);
-    a.moeFirstExpert = c.moeFirstExpert; a.moeNumLocal = c.moeNumLocal; a.moeScratch = e.g.moeScratch; a.moeCounters = e.g.moeCounters;
+    a.moeFirstExpert = c.moeFirstExpert; a.moeNumLocal = c.moeNumLocal; a.moeScratch = e.b.moeScratch; a.moeCounters = e.b.moeCounters;
     if (fusedAr) fillAr(e, a.ar, 1);
     { const int r = gemvQ40Tma(PRO_PLAIN_, EPI_MOE_DOWN_, 1, a, c.numSms, stream, pdl); if (r != 0) return r == 1 ? -32 : r; }
     return 0;
@@ -127,20 +184,20 @@ static int engineDecodeMega(Engine &e, bool greedyAdvance, cudaStream_t stream) 
     if (!e.megaLayers || c.nExperts > 0 || c.wType != 0) return 1;
     MegaArgs m{};
     m.layers = e.megaLayers; m.nLayers = c.nLayers; m.dim = c.dim; m.nHeads = c.nHeads; m.nKvHeads = c.nKvHeads; m.headDim = c.headDim;
-    m.ffDim = c.ffDim; m.vocab = c.vocab; m.vocabFull = e.g.vocabFull; m.seqLen = c.seqLen; m.nSplits = c.nSplits; m.eps = c.eps;
+    m.ffDim = c.ffDim; m.vocab = c.vocab; m.vocabFull = c.vocabFull; m.seqLen = c.seqLen; m.nSplits = c.nSplits; m.eps = c.eps;
     m.embedding = embTable(e); m.finalNorm = e.g.finalNorm; m.rope = e.g.rope;
     m.wclsQs = (const uint8_t *)e.g.wclsQs; m.wclsSc = (const uint8_t *)e.g.wclsSc;
-    m.tokens = e.g.tokens; m.pos = e.g.pos; m.history = e.g.history;
-    m.logits = e.g.logits; m.maxInflight = e.megaInflight;
+    m.tokens = e.b.tokens; m.pos = e.b.pos; m.history = e.b.history;
+    m.logits = e.b.logits; m.maxInflight = e.megaInflight;
     m.xW = e.megaX; m.xW2 = e.megaX2; m.flags = e.megaFlags; m.qkvW = e.megaQkv; m.zW = e.megaZ; m.hF = (float *)e.megaH; m.launchSeq = e.megaSeq; m.abortFlag = e.abortDev;
-    m.syncNs = (e.comm.nRanks > 1 && e.megaSeq) ? (unsigned long long *)(e.megaSeq + 2) : nullptr;
-    m.attnPartial = e.g.attnPartial; m.attnCounters = e.g.attnCounters;
-    m.argVal = e.g.argVal; m.argIdx = e.g.argIdx; m.argCounter = e.g.argCounter; m.gridCounter = e.megaCounter;
+    m.syncNs = (e.tp && e.megaSeq) ? (unsigned long long *)(e.megaSeq + 2) : nullptr;
+    m.attnPartial = e.b.attnPartial; m.attnCounters = e.b.attnCounters;
+    m.argVal = e.b.argVal; m.argIdx = e.b.argIdx; m.argCounter = e.b.argCounter; m.gridCounter = e.megaCounter;
     m.rowOffsetGlobal = c.rank * c.vocab; m.greedyAdvance = greedyAdvance ? 1u : 0u; m.vocabLimit = e.vocabLimit;
     m.trace = e.trace;
     m.traceCtas = e.traceAllCtas ? c.numSms : 1u;
     m.traceStride = e.traceAllCtas ? (uint32_t)(((size_t)e.traceCap * 4) / c.numSms) : 0u;
-    if (e.comm.nRanks > 1) fillAr(e, m.ar, 0);
+    if (e.tp) fillAr(e, m.ar, 0);
     return launchMegaDecode(m, (int)(e.megaCtas ? e.megaCtas : c.numSms), stream);
 }
 
@@ -163,94 +220,94 @@ static int engineForward(Engine &e, int nb, int logitsMode, bool greedyAdvance, 
     uint32_t slot = 0;
     auto nextTrace = [&]() -> uint64_t * { uint64_t *t = (e.trace && slot < e.traceCap) ? e.trace + (size_t)slot * 4 : nullptr; slot++; return t; };
 
-    DL_TRY(launchEmbedding(embTable(e), e.g.tokens, e.g.x, c.dim, c.dim, e.g.vocabFull, nb, stream));
+    DL_TRY(launchEmbedding(embTable(e), e.b.tokens, e.b.x, c.dim, c.dim, c.vocabFull, nb, stream));
     for (uint32_t l = 0; l < c.nLayers; l++) {
         const LayerPtrs &L = e.layers[l];
         GemvArgs a{};
         // 1. rmsnorm -> q80 -> QKV
         a.qs = (const uint32_t *)L.qkvQs; a.scales = (const __half *)L.qkvSc; a.d = qkvDim; a.n = c.dim;
-        a.in = e.g.x; a.inStride = c.dim; a.normW = L.norm0; a.eps = c.eps; a.out = e.g.qkv; a.outStride = qkvDim; a.trace = nextTrace();
+        a.in = e.b.x; a.inStride = c.dim; a.normW = L.norm0; a.eps = c.eps; a.out = e.b.qkv; a.outStride = qkvDim; a.trace = nextTrace();
         DL_TRY(gemvSel(e, PRO_RMSNORM_, EPI_STORE_, nb, a, c.numSms, stream, pdl));
         if (nb == 1 && e.fusedAttn) {
             // 2+3. qk-norm + rope + kv append + attention in one launch
             AttnFusedArgs f{};
-            f.qkv = e.g.qkv; f.pos = e.g.pos; f.rope = e.g.rope; f.qNorm = L.qNorm; f.kNorm = L.kNorm; f.eps = c.eps;
-            f.kCache = (__nv_bfloat16 *)L.kCache; f.vCache = (__nv_bfloat16 *)L.vCache;
+            f.qkv = e.b.qkv; f.pos = e.b.pos; f.rope = e.g.rope; f.qNorm = L.qNorm; f.kNorm = L.kNorm; f.eps = c.eps;
+            f.kCache = (__nv_bfloat16 *)e.kCache[l]; f.vCache = (__nv_bfloat16 *)e.vCache[l];
             f.nHeads = c.nHeads; f.nKvHeads = c.nKvHeads; f.headDim = c.headDim; f.seqLen = c.seqLen; f.nSplits = c.nSplits;
-            f.partial = e.g.attnPartial; f.counters = e.g.attnCounters; f.out = e.g.z; f.trace = nextTrace();
+            f.partial = e.b.attnPartial; f.counters = e.b.attnCounters; f.out = e.b.z; f.trace = nextTrace();
             DL_TRY(launchAttnFused(f, stream, pdl));
         } else {
             // 2. qk-norm + rope + kv write
             RopeKvArgs r{};
-            r.qkv = e.g.qkv; r.qkvStride = qkvDim; r.pos = e.g.pos; r.rope = e.g.rope; r.qNorm = L.qNorm; r.kNorm = L.kNorm;
+            r.qkv = e.b.qkv; r.qkvStride = qkvDim; r.pos = e.b.pos; r.rope = e.g.rope; r.qNorm = L.qNorm; r.kNorm = L.kNorm;
             r.eps = c.eps; r.nHeads = c.nHeads; r.nKvHeads = c.nKvHeads; r.headDim = c.headDim; r.seqLen = c.seqLen;
-            r.kCache = (__nv_bfloat16 *)L.kCache; r.vCache = (__nv_bfloat16 *)L.vCache;
+            r.kCache = (__nv_bfloat16 *)e.kCache[l]; r.vCache = (__nv_bfloat16 *)e.vCache[l];
             DL_TRY(launchRopeKv(r, nb, stream, pdl));
             // 3. attention
             AttnArgs t{};
-            t.qkv = e.g.qkv; t.qkvStride = qkvDim; t.pos = e.g.pos; t.kCache = r.kCache; t.vCache = r.vCache;
+            t.qkv = e.b.qkv; t.qkvStride = qkvDim; t.pos = e.b.pos; t.kCache = r.kCache; t.vCache = r.vCache;
             t.nHeads = c.nHeads; t.nKvHeads = c.nKvHeads; t.headDim = c.headDim; t.seqLen = c.seqLen; t.nSplits = c.nSplits;
-            t.partial = e.g.attnPartial; t.counters = e.g.attnCounters; t.out = e.g.z; t.outStride = qDim;
+            t.partial = e.b.attnPartial; t.counters = e.b.attnCounters; t.out = e.b.z; t.outStride = qDim;
             DL_TRY(launchAttnDecode(t, nb, stream, pdl));
         }
         // 4. q80 -> WO, residual add
         a = GemvArgs{};
         a.qs = (const uint32_t *)L.woQs; a.scales = (const __half *)L.woSc; a.d = c.dim; a.n = qDim;
-        a.in = e.g.z; a.inStride = qDim; a.out = e.g.x; a.outStride = c.dim; a.trace = nextTrace();
-        if (e.comm.nRanks > 1) fillAr(e, a.ar, 0);
+        a.in = e.b.z; a.inStride = qDim; a.out = e.b.x; a.outStride = c.dim; a.trace = nextTrace();
+        if (e.tp) fillAr(e, a.ar, 0);
         DL_TRY(gemvSel(e, PRO_PLAIN_, EPI_RESIDUAL_, nb, a, c.numSms, stream, pdl));
         if (c.nExperts > 0) {
             // 5-7. mixture of experts: router -> k x (W1|W3 -> silu*up) -> k x W2, weighted sum, residual (+ all-reduce)
             if (nb != 1) return -13;
             nextTrace();
             uint64_t *t13 = nextTrace(), *t2 = nextTrace();
-            DL_TRY(runMoe(e, L, e.g.x, e.comm.nRanks > 1, t13, t2, stream, pdl));
+            DL_TRY(runMoe(e, L, e.b.x, e.tp, t13, t2, stream, pdl));
             continue;
         }
         // 5. rmsnorm -> q80 -> W1|W3 -> silu*up
         a = GemvArgs{};
         a.qs = (const uint32_t *)L.w13Qs; a.scales = (const __half *)L.w13Sc; a.d = 2 * c.ffDim; a.n = c.dim;
-        a.in = e.g.x; a.inStride = c.dim; a.normW = L.norm1; a.eps = c.eps; a.out = e.g.h; a.outStride = c.ffDim; a.trace = nextTrace();
+        a.in = e.b.x; a.inStride = c.dim; a.normW = L.norm1; a.eps = c.eps; a.out = e.b.h; a.outStride = c.ffDim; a.trace = nextTrace();
         DL_TRY(gemvSel(e, PRO_RMSNORM_, EPI_SWIGLU_, nb, a, c.numSms, stream, pdl));
         // 6. q80 -> W2, residual add
         a = GemvArgs{};
         a.qs = (const uint32_t *)L.w2Qs; a.scales = (const __half *)L.w2Sc; a.d = c.dim; a.n = c.ffDim;
-        a.in = e.g.h; a.inStride = c.ffDim; a.out = e.g.x; a.outStride = c.dim; a.trace = nextTrace();
-        if (e.comm.nRanks > 1) fillAr(e, a.ar, 1);
+        a.in = e.b.h; a.inStride = c.ffDim; a.out = e.b.x; a.outStride = c.dim; a.trace = nextTrace();
+        if (e.tp) fillAr(e, a.ar, 1);
         DL_TRY(gemvSel(e, PRO_PLAIN_, EPI_RESIDUAL_, nb, a, c.numSms, stream, pdl));
     }
     if (logitsMode != 0) {
         GemvArgs a{};
         a.qs = (const uint32_t *)e.g.wclsQs; a.scales = (const __half *)e.g.wclsSc; a.d = c.vocab; a.n = c.dim;
-        a.normW = e.g.finalNorm; a.eps = c.eps; a.inStride = c.dim; a.outStride = c.vocab; a.out = e.g.logits; a.trace = nextTrace();
+        a.normW = e.g.finalNorm; a.eps = c.eps; a.inStride = c.dim; a.outStride = c.vocab; a.out = e.b.logits; a.trace = nextTrace();
         if (logitsMode == 1) {
-            a.in = e.g.x + (size_t)(nb - 1) * c.dim;
+            a.in = e.b.x + (size_t)(nb - 1) * c.dim;
             int r = 1;
             if (greedyAdvance && e.fusedArgmax && c.wType == 0) {
                 // logits + greedy sampling + position advance in one launch
-                a.argVal = e.g.argVal; a.argIdx = e.g.argIdx; a.argCounter = e.g.argCounter;
-                a.tokenOut = e.g.tokens; a.posInOut = e.g.pos; a.history = e.g.history; a.historyCap = c.seqLen;
+                a.argVal = e.b.argVal; a.argIdx = e.b.argIdx; a.argCounter = e.b.argCounter;
+                a.tokenOut = e.b.tokens; a.posInOut = e.b.pos; a.history = e.b.history; a.historyCap = c.seqLen;
                 a.rowOffsetGlobal = c.rank * c.vocab; a.vocabLimit = e.vocabLimit;
-                if (e.comm.nRanks > 1) fillAr(e, a.ar, 0);
+                if (e.tp) fillAr(e, a.ar, 0);
                 r = gemvQ40Tma(PRO_RMSNORM_, EPI_ARGMAX_, 1, a, c.numSms, stream, pdl);
                 if (r < 0) return r;
             }
             if (r == 1) {
                 // the stand-alone arg-max kernel sees this rank's vocabulary slice only: under tensor parallelism the ranks would
                 // pick different (local) ids, so the non-fused route is refused there instead of silently diverging
-                if (greedyAdvance && e.comm.nRanks > 1) return -33;
+                if (greedyAdvance && e.tp) return -33;
                 a.argVal = nullptr; a.argIdx = nullptr; a.argCounter = nullptr; a.tokenOut = nullptr; a.posInOut = nullptr; a.history = nullptr;
                 a.ar = ArArgs{};
                 DL_TRY(gemvSel(e, PRO_RMSNORM_, EPI_STORE_, 1, a, c.numSms, stream, pdl));
                 if (greedyAdvance)
-                    DL_TRY(launchArgmaxAdvance(e.g.logits, localVocabLimit(e), e.g.tokens, e.g.pos, e.g.history, c.seqLen, stream, pdl));
+                    DL_TRY(launchArgmaxAdvance(e.b.logits, localVocabLimit(e), e.b.tokens, e.b.pos, e.b.history, c.seqLen, stream, pdl));
             }
         } else {
-            a.in = e.g.x;
+            a.in = e.b.x;
             DL_TRY(gemvSel(e, PRO_RMSNORM_, EPI_STORE_, nb, a, c.numSms, stream, pdl));
             if (greedyAdvance) {
-                if (e.comm.nRanks > 1) return -33;
-                DL_TRY(launchArgmaxAdvance(e.g.logits, localVocabLimit(e), e.g.tokens, e.g.pos, e.g.history, c.seqLen, stream, pdl));
+                if (e.tp) return -33;
+                DL_TRY(launchArgmaxAdvance(e.b.logits, localVocabLimit(e), e.b.tokens, e.b.pos, e.b.history, c.seqLen, stream, pdl));
             }
         }
     }
@@ -261,58 +318,59 @@ static int engineForward(Engine &e, int nb, int logitsMode, bool greedyAdvance, 
 static int enginePrefill(Engine &e, uint32_t T, uint32_t p0, int wantLogits, cudaStream_t stream) {
     const EngineConfig &c = e.cfg;
     const GlobalPtrs &g = e.g;
+    const Buffers &b = e.b;
     const bool pdl = c.usePdl != 0;   // every kernel of this chain waits (griddepcontrol.wait) before touching its predecessor's data
     const uint32_t qDim = c.nHeads * c.headDim, kvDim = c.nKvHeads * c.headDim, qkvDim = qDim + 2 * kvDim;
-    if (T < 1 || T > g.maxPrefill || T > 256) return -11;
+    if (T < 1 || T > c.maxPrefill) return -11;
     if (c.wType != 0) return -35;   // tensor-core path: q40 matrices
-    const bool tp = e.comm.nRanks > 1;
+    const bool tp = e.tp;
     ArArgs arP{};
     if (tp) {
-        if (e.comm.prefillSlotStride < T * c.dim) return -12;
         fillAr(e, arP, 0);
-        arP.slotStride = e.comm.prefillSlotStride;
-        for (uint32_t r = 0; r < e.comm.nRanks; r++) arP.slots[r] = (uint64_t *)((uint8_t *)e.comm.arena[r] + e.comm.prefillSlotsOff);
-        arP.slotsMc = e.comm.mcArena ? (uint64_t *)((uint8_t *)e.comm.mcArena + e.comm.prefillSlotsOff) : nullptr;
+        const uint64_t off = arenaLayout(c).prefillSlotsOff;
+        arP.slotStride = c.maxPrefill * c.dim;
+        for (uint32_t r = 0; r < c.nRanks; r++) arP.slots[r] = (uint64_t *)((uint8_t *)e.comm.arena[r] + off);
+        arP.slotsMc = e.comm.mcArena ? (uint64_t *)((uint8_t *)e.comm.mcArena + off) : nullptr;
     }
-    DL_TRY(launchEmbedding(embTable(e), g.pTokens, g.px, c.dim, c.dim, g.vocabFull, (int)T, stream));
+    DL_TRY(launchEmbedding(embTable(e), b.pTokens, b.px, c.dim, c.dim, c.vocabFull, (int)T, stream));
     for (uint32_t l = 0; l < c.nLayers; l++) {
         const LayerPtrs &L = e.layers[l];
-        DL_TRY(launchRmsNormBf16(g.px, c.dim, L.norm0, g.pxn, c.dim, c.dim, c.eps, T, stream, pdl));
-        DL_TRY(gemmQ40Tc(GEPI_STORE_F32_, L.qkvQs, L.qkvSc, qkvDim, c.dim, g.pxn, c.dim, T, g.pqkv, qkvDim, c.numSms, stream, pdl));
+        DL_TRY(launchRmsNormBf16(b.px, c.dim, L.norm0, b.pxn, c.dim, c.dim, c.eps, T, stream, pdl));
+        DL_TRY(gemmQ40Tc(GEPI_STORE_F32_, L.qkvQs, L.qkvSc, qkvDim, c.dim, b.pxn, c.dim, T, b.pqkv, qkvDim, c.numSms, stream, pdl));
         RopeKvArgs r{};
-        r.qkv = g.pqkv; r.qkvStride = qkvDim; r.pos = g.pPos; r.rope = g.rope; r.qNorm = L.qNorm; r.kNorm = L.kNorm;
+        r.qkv = b.pqkv; r.qkvStride = qkvDim; r.pos = b.pPos; r.rope = g.rope; r.qNorm = L.qNorm; r.kNorm = L.kNorm;
         r.eps = c.eps; r.nHeads = c.nHeads; r.nKvHeads = c.nKvHeads; r.headDim = c.headDim; r.seqLen = c.seqLen;
-        r.kCache = (__nv_bfloat16 *)L.kCache; r.vCache = (__nv_bfloat16 *)L.vCache;
+        r.kCache = (__nv_bfloat16 *)e.kCache[l]; r.vCache = (__nv_bfloat16 *)e.vCache[l];
         DL_TRY(launchRopeKv(r, (int)T, stream, pdl));
         int attnRc = 1;
         if (e.tcAttn) {
             // tensor-core attention over the whole chunk: the tokens of a chunk sit at consecutive positions p0 .. p0 + T - 1
             AttnPrefillArgs ap{};
-            ap.qkv = g.pqkv; ap.qkvStride = qkvDim; ap.T = T; ap.p0 = p0; ap.nHeads = c.nHeads; ap.nKvHeads = c.nKvHeads;
+            ap.qkv = b.pqkv; ap.qkvStride = qkvDim; ap.T = T; ap.p0 = p0; ap.nHeads = c.nHeads; ap.nKvHeads = c.nKvHeads;
             ap.headDim = c.headDim; ap.seqLen = c.seqLen; ap.kCache = r.kCache; ap.vCache = r.vCache;
-            ap.out = (__nv_bfloat16 *)g.pzb; ap.outStride = qDim;
+            ap.out = (__nv_bfloat16 *)b.pzb; ap.outStride = qDim;
             attnRc = launchAttnPrefillTc(ap, stream, pdl);
             if (attnRc < 0) return attnRc;
         }
         if (attnRc == 1) {
             AttnArgs t{};
-            t.qkv = g.pqkv; t.qkvStride = qkvDim; t.pos = g.pPos; t.kCache = r.kCache; t.vCache = r.vCache;
+            t.qkv = b.pqkv; t.qkvStride = qkvDim; t.pos = b.pPos; t.kCache = r.kCache; t.vCache = r.vCache;
             t.nHeads = c.nHeads; t.nKvHeads = c.nKvHeads; t.headDim = c.headDim; t.seqLen = c.seqLen; t.nSplits = 1;
-            t.partial = g.pAttnPartial; t.counters = g.pAttnCounters; t.out = nullptr; t.outStride = qDim; t.outBf16 = (__nv_bfloat16 *)g.pzb;
+            t.partial = b.pAttnPartial; t.counters = b.pAttnCounters; t.out = nullptr; t.outStride = qDim; t.outBf16 = (__nv_bfloat16 *)b.pzb;
             DL_TRY(launchAttnDecode(t, (int)T, stream, pdl));
         }
         // tensor parallel: partial product into the (now free) qkv buffer with all SMs / split-K, then all-reduce + residual over
         // peer memory as its own kernel (DL_PREFILL_FUSED_AR=1: the one-kernel GEMM + all-reduce epilogue instead)
         if (tp && !e.prefillFusedAr) {
             arP.parity = 0;
-            DL_TRY(gemmQ40Tc(GEPI_STORE_F32_, L.woQs, L.woSc, c.dim, qDim, g.pzb, qDim, T, g.pqkv, c.dim, c.numSms, stream, pdl));
-            DL_TRY(launchArResidual(g.px, g.pqkv, c.dim, T, arP, stream, pdl));
-        } else if (tp) { arP.parity = 0; DL_TRY(gemmQ40TcAr(L.woQs, L.woSc, c.dim, qDim, g.pzb, qDim, T, g.px, c.dim, c.numSms, stream, arP)); }
-        else DL_TRY(gemmQ40Tc(GEPI_RESIDUAL_, L.woQs, L.woSc, c.dim, qDim, g.pzb, qDim, T, g.px, c.dim, c.numSms, stream, pdl));
+            DL_TRY(gemmQ40Tc(GEPI_STORE_F32_, L.woQs, L.woSc, c.dim, qDim, b.pzb, qDim, T, b.pqkv, c.dim, c.numSms, stream, pdl));
+            DL_TRY(launchArResidual(b.px, b.pqkv, c.dim, T, arP, stream, pdl));
+        } else if (tp) { arP.parity = 0; DL_TRY(gemmQ40TcAr(L.woQs, L.woSc, c.dim, qDim, b.pzb, qDim, T, b.px, c.dim, c.numSms, stream, arP)); }
+        else DL_TRY(gemmQ40Tc(GEPI_RESIDUAL_, L.woQs, L.woSc, c.dim, qDim, b.pzb, qDim, T, b.px, c.dim, c.numSms, stream, pdl));
         if (c.nExperts > 0) {
             // mixture of experts: route the whole chunk, sort the (token, expert) pairs, grouped tensor-core GEMMs, weighted combine
             MoePrefillArgs mo{};
-            mo.x = g.px; mo.xnScratch = g.pxn; mo.norm = L.norm1; mo.gate = L.moeGate; mo.w13Qs = L.w13Qs; mo.w13Sc = L.w13Sc;
+            mo.x = b.px; mo.xnScratch = b.pxn; mo.norm = L.norm1; mo.gate = L.moeGate; mo.w13Qs = L.w13Qs; mo.w13Sc = L.w13Sc;
             mo.w2Qs = L.w2Qs; mo.w2Sc = L.w2Sc; mo.T = T; mo.dim = c.dim; mo.ff = c.ffDim; mo.nExperts = c.nExperts; mo.k = c.nActiveExperts;
             mo.firstLocal = c.moeFirstExpert; mo.nLocal = c.moeNumLocal; mo.eps = c.eps; mo.numSms = (int)c.numSms;
             if (tp) { arP.parity = 1; mo.ar = arP; }
@@ -320,23 +378,59 @@ static int enginePrefill(Engine &e, uint32_t T, uint32_t p0, int wantLogits, cud
             if (mr != 0) return mr == 1 ? -36 : mr;
             continue;
         }
-        DL_TRY(launchRmsNormBf16(g.px, c.dim, L.norm1, g.pxn, c.dim, c.dim, c.eps, T, stream, pdl));
-        DL_TRY(gemmQ40Tc(GEPI_SWIGLU_BF16_, L.w13Qs, L.w13Sc, 2 * c.ffDim, c.dim, g.pxn, c.dim, T, g.phb, c.ffDim, c.numSms, stream, pdl));
+        DL_TRY(launchRmsNormBf16(b.px, c.dim, L.norm1, b.pxn, c.dim, c.dim, c.eps, T, stream, pdl));
+        DL_TRY(gemmQ40Tc(GEPI_SWIGLU_BF16_, L.w13Qs, L.w13Sc, 2 * c.ffDim, c.dim, b.pxn, c.dim, T, b.phb, c.ffDim, c.numSms, stream, pdl));
         if (tp && !e.prefillFusedAr) {
             arP.parity = 1;
-            DL_TRY(gemmQ40Tc(GEPI_STORE_F32_, L.w2Qs, L.w2Sc, c.dim, c.ffDim, g.phb, c.ffDim, T, g.pqkv, c.dim, c.numSms, stream, pdl));
-            DL_TRY(launchArResidual(g.px, g.pqkv, c.dim, T, arP, stream, pdl));
-        } else if (tp) { arP.parity = 1; DL_TRY(gemmQ40TcAr(L.w2Qs, L.w2Sc, c.dim, c.ffDim, g.phb, c.ffDim, T, g.px, c.dim, c.numSms, stream, arP)); }
-        else DL_TRY(gemmQ40Tc(GEPI_RESIDUAL_, L.w2Qs, L.w2Sc, c.dim, c.ffDim, g.phb, c.ffDim, T, g.px, c.dim, c.numSms, stream, pdl));
+            DL_TRY(gemmQ40Tc(GEPI_STORE_F32_, L.w2Qs, L.w2Sc, c.dim, c.ffDim, b.phb, c.ffDim, T, b.pqkv, c.dim, c.numSms, stream, pdl));
+            DL_TRY(launchArResidual(b.px, b.pqkv, c.dim, T, arP, stream, pdl));
+        } else if (tp) { arP.parity = 1; DL_TRY(gemmQ40TcAr(L.w2Qs, L.w2Sc, c.dim, c.ffDim, b.phb, c.ffDim, T, b.px, c.dim, c.numSms, stream, arP)); }
+        else DL_TRY(gemmQ40Tc(GEPI_RESIDUAL_, L.w2Qs, L.w2Sc, c.dim, c.ffDim, b.phb, c.ffDim, T, b.px, c.dim, c.numSms, stream, pdl));
     }
     if (wantLogits) {
         GemvArgs a{};
         a.qs = (const uint32_t *)g.wclsQs; a.scales = (const __half *)g.wclsSc; a.d = c.vocab; a.n = c.dim;
-        a.normW = g.finalNorm; a.eps = c.eps; a.inStride = c.dim; a.outStride = c.vocab; a.out = g.logits;
-        a.in = g.px + (size_t)(T - 1) * c.dim;
+        a.normW = g.finalNorm; a.eps = c.eps; a.inStride = c.dim; a.outStride = c.vocab; a.out = b.logits;
+        a.in = b.px + (size_t)(T - 1) * c.dim;
         DL_TRY(gemvSel(e, PRO_RMSNORM_, EPI_STORE_, 1, a, c.numSms, stream, false));
     }
     return 0;
+}
+
+// Allocates and zeroes the working buffers and KV caches on the current device, finished before it returns: a forward may
+// read cache rows that no kernel has written yet.
+static bool allocBuffers(Engine &e) {
+    const EngineConfig &c = e.cfg;
+    bool ok = true;
+    auto zeroed = [&](size_t bytes) -> void * {
+        void *p = nullptr;
+        if (!ok || bytes == 0) return nullptr;
+        if (cudaMalloc(&p, bytes) != cudaSuccess) { ok = false; return nullptr; }
+        e.owned.push_back(p);
+        ok = cudaMemset(p, 0, bytes) == cudaSuccess;
+        return p;
+    };
+    const size_t mb = c.maxBatch, mp = c.maxPrefill, dim = c.dim, ff = c.ffDim, heads = c.nHeads, hd = c.headDim;
+    const size_t kAct = std::max(1u, c.nActiveExperts), qDim = heads * hd, qkvDim = qDim + 2 * (size_t)c.nKvHeads * hd;
+    Buffers &b = e.b;
+    b.tokens = (int *)zeroed(mb * 4); b.pos = (int *)zeroed(mb * 4);
+    b.x = (float *)zeroed(mb * dim * 4); b.qkv = (float *)zeroed(mb * qkvDim * 4); b.z = (float *)zeroed(mb * qDim * 4);
+    b.h = (float *)zeroed(std::max(mb, kAct) * ff * 4); b.logits = (float *)zeroed(mb * c.vocab * 4);
+    b.attnPartial = (float *)zeroed(mb * heads * c.nSplits * (hd + 2) * 4); b.attnCounters = (unsigned int *)zeroed(mb * heads * 4);
+    b.history = (int *)zeroed(((size_t)c.seqLen + 1) * 4);
+    b.expertIdx = (int *)zeroed(mb * kAct * 4); b.expertWeight = (float *)zeroed(mb * kAct * 4);
+    b.routerLogits = (float *)zeroed(mb * std::max(1u, c.nExperts) * 4); b.routerCounter = (unsigned int *)zeroed(mb * 4);
+    b.moeScratch = (float *)zeroed(kAct * dim * 4); b.moeCounters = (unsigned int *)zeroed(256 * 4);
+    b.pTokens = (int *)zeroed(mp * 4); b.pPos = (int *)zeroed(mp * 4);
+    b.px = (float *)zeroed(mp * dim * 4); b.pqkv = (float *)zeroed(mp * std::max(qkvDim, dim) * 4);
+    b.pxn = zeroed(mp * dim * 2); b.pzb = zeroed(mp * qDim * 2); b.phb = zeroed(mp * ff * 2);
+    b.pAttnPartial = (float *)zeroed(mp * heads * (hd + 2) * 4); b.pAttnCounters = (unsigned int *)zeroed(mp * heads * 4);
+    b.argVal = (float *)zeroed(256 * 4); b.argIdx = (int *)zeroed(256 * 4); b.argCounter = (unsigned int *)zeroed(4 * 4);
+    for (uint32_t l = 0; l < c.nLayers; l++) {
+        e.kCache.push_back(zeroed((size_t)c.nKvHeads * c.seqLen * hd * 2));
+        e.vCache.push_back(zeroed((size_t)c.nKvHeads * c.seqLen * hd * 2));
+    }
+    return ok && cudaDeviceSynchronize() == cudaSuccess;
 }
 
 }  // namespace dl
@@ -345,7 +439,7 @@ using dl::Engine;
 
 DL_EXPORT void *dl_engine_create(const dl::EngineConfig *cfg) {
     Engine *e = new Engine();
-    e->cfg = *cfg;
+    e->cfg = dl::applyLimits(*cfg);
     dl::gHiddenAct = cfg->hiddenAct;
     e->layers.resize(cfg->nLayers);
     e->fusedAttn = std::getenv("DL_NO_FUSED_ATTN") == nullptr;
@@ -359,6 +453,11 @@ DL_EXPORT void *dl_engine_create(const dl::EngineConfig *cfg) {
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         e->cfg.numSms = (uint32_t)sms;
     }
+    if (e->cfg.nSplits == 0) e->cfg.nSplits = std::max(1u, std::min(32u, 2 * e->cfg.numSms / std::max(1u, e->cfg.nHeads)));
+    if (!dl::allocBuffers(*e)) {
+        dl_engine_destroy(e);
+        return nullptr;
+    }
     return e;
 }
 
@@ -371,6 +470,7 @@ DL_EXPORT void dl_engine_destroy(void *h) {
     if (e->megaCounter) cudaFree(e->megaCounter);
     for (void *q : {(void *)e->megaX, (void *)e->megaX2, (void *)e->megaQkv, (void *)e->megaZ, (void *)e->megaH, (void *)e->megaSeq}) if (q) cudaFree(q);
     if (e->abortHost) cudaFreeHost(e->abortHost);
+    for (void *p : e->owned) cudaFree(p);
     delete e;
 }
 
@@ -386,6 +486,20 @@ DL_EXPORT int dl_engine_set_globals(void *h, const dl::GlobalPtrs *p) {
     return 0;
 }
 
+DL_EXPORT int dl_engine_get_config(void *h, dl::EngineConfig *cfg) {
+    *cfg = ((Engine *)h)->cfg;
+    return 0;
+}
+
+DL_EXPORT int dl_engine_buffers(void *h, dl::EngineBuffers *out) {
+    const Engine *e = (Engine *)h;
+    const dl::Buffers &b = e->b;
+    *out = dl::EngineBuffers{b.tokens, b.pos, b.history, b.logits, b.x, b.pTokens, b.pPos, e->kCache.data(), e->vCache.data()};
+    return 0;
+}
+
+DL_EXPORT size_t dl_engine_arena_bytes(const dl::EngineConfig *cfg) { return dl::arenaLayout(dl::applyLimits(*cfg)).bytes; }
+
 // Uploads the per-layer pointer table and switches single-token forwards to the persistent kernel.
 DL_EXPORT int dl_engine_enable_mega(void *h, int enable) {
     Engine *e = (Engine *)h;
@@ -397,7 +511,7 @@ DL_EXPORT int dl_engine_enable_mega(void *h, int enable) {
             m.qkvQs = (const uint8_t *)L.qkvQs; m.qkvSc = (const uint8_t *)L.qkvSc; m.woQs = (const uint8_t *)L.woQs; m.woSc = (const uint8_t *)L.woSc;
             m.w13Qs = (const uint8_t *)L.w13Qs; m.w13Sc = (const uint8_t *)L.w13Sc; m.w2Qs = (const uint8_t *)L.w2Qs; m.w2Sc = (const uint8_t *)L.w2Sc;
             m.norm0 = L.norm0; m.norm1 = L.norm1; m.qNorm = L.qNorm; m.kNorm = L.kNorm;
-            m.kCache = (__nv_bfloat16 *)L.kCache; m.vCache = (__nv_bfloat16 *)L.vCache;
+            m.kCache = (__nv_bfloat16 *)e->kCache[l]; m.vCache = (__nv_bfloat16 *)e->vCache[l];
         }
         DL_CUDA_CHECK(cudaMalloc(&e->megaLayers, tab.size() * sizeof(dl::MegaLayer)));
         DL_CUDA_CHECK(cudaMemcpy(e->megaLayers, tab.data(), tab.size() * sizeof(dl::MegaLayer), cudaMemcpyHostToDevice));
@@ -462,12 +576,13 @@ DL_EXPORT int dl_engine_sampler_seed(void *h, unsigned long long seed) {
         DL_CUDA_CHECK(cudaMemset(e->gatherEpoch, 0, 64));
         DL_CUDA_CHECK(cudaMalloc(&e->gatherBlockCounter, 64));
         DL_CUDA_CHECK(cudaMemset(e->gatherBlockCounter, 0, 64));
-        if (e->comm.nRanks > 1) {
+        if (e->tp) {
+            const dl::ArenaLayout L = dl::arenaLayout(c);
             float *g[dl::kApiMaxRanks] = {};
             unsigned int *f[dl::kApiMaxRanks] = {};
-            for (uint32_t r = 0; r < e->comm.nRanks; r++) {
-                g[r] = (float *)((uint8_t *)e->comm.arena[r] + e->comm.gatherOff);
-                f[r] = (unsigned int *)((uint8_t *)e->comm.arena[r] + e->comm.flagsOff);
+            for (uint32_t r = 0; r < c.nRanks; r++) {
+                g[r] = (float *)((uint8_t *)e->comm.arena[r] + L.gatherOff);
+                f[r] = (unsigned int *)((uint8_t *)e->comm.arena[r] + L.flagsOff);
             }
             DL_CUDA_CHECK(cudaMalloc(&e->gatherUcDev, sizeof(g)));
             DL_CUDA_CHECK(cudaMalloc(&e->flagUcDev, sizeof(f)));
@@ -487,24 +602,27 @@ DL_EXPORT int dl_engine_sample(void *h, float temperature, float topp, cudaStrea
     Engine *e = (Engine *)h;
     const dl::EngineConfig &c = e->cfg;
     if (!e->rngState) return -50;
-    const uint32_t nR = e->comm.nRanks > 1 ? e->comm.nRanks : 1;
+    const uint32_t nR = e->tp ? c.nRanks : 1;
     const uint32_t full = c.vocab * nR;
     const uint32_t n = (e->vocabLimit && e->vocabLimit < full) ? e->vocabLimit : full;
     if (nR == 1)
-        return dl::launchSample(e->g.logits, e->probScratch, n, temperature, topp, e->rngState, e->g.tokens, e->g.pos, e->g.history, c.seqLen,
+        return dl::launchSample(e->b.logits, e->probScratch, n, temperature, topp, e->rngState, e->b.tokens, e->b.pos, e->b.history, c.seqLen,
                                 nullptr, nullptr, 1, stream);
-    uint8_t *mine = (uint8_t *)e->comm.arena[e->comm.rank];
-    float *gatherLocal = (float *)(mine + e->comm.gatherOff);
-    unsigned int *flagLocal = (unsigned int *)(mine + e->comm.flagsOff);
-    float *gatherMc = e->comm.mcArena ? (float *)((uint8_t *)e->comm.mcArena + e->comm.gatherOff) : nullptr;
-    unsigned int *flagMc = e->comm.mcArena ? (unsigned int *)((uint8_t *)e->comm.mcArena + e->comm.flagsOff) : nullptr;
-    DL_TRY(dl::launchLogitsGather(e->g.logits, c.vocab, c.rank, nR, gatherMc, e->gatherUcDev, flagMc, e->flagUcDev, e->gatherBlockCounter, stream));
-    return dl::launchSample(gatherLocal, e->probScratch, n, temperature, topp, e->rngState, e->g.tokens, e->g.pos, e->g.history, c.seqLen, flagLocal,
+    const dl::ArenaLayout L = dl::arenaLayout(c);
+    uint8_t *mine = (uint8_t *)e->comm.arena[c.rank];
+    float *gatherLocal = (float *)(mine + L.gatherOff);
+    unsigned int *flagLocal = (unsigned int *)(mine + L.flagsOff);
+    float *gatherMc = e->comm.mcArena ? (float *)((uint8_t *)e->comm.mcArena + L.gatherOff) : nullptr;
+    unsigned int *flagMc = e->comm.mcArena ? (unsigned int *)((uint8_t *)e->comm.mcArena + L.flagsOff) : nullptr;
+    DL_TRY(dl::launchLogitsGather(e->b.logits, c.vocab, c.rank, nR, gatherMc, e->gatherUcDev, flagMc, e->flagUcDev, e->gatherBlockCounter, stream));
+    return dl::launchSample(gatherLocal, e->probScratch, n, temperature, topp, e->rngState, e->b.tokens, e->b.pos, e->b.history, c.seqLen, flagLocal,
                             e->gatherEpoch, nR, stream);
 }
 
 DL_EXPORT int dl_engine_set_comm(void *h, const dl::CommPtrs *p) {
-    ((Engine *)h)->comm = *p;
+    Engine *e = (Engine *)h;
+    e->comm = *p;
+    e->tp = e->cfg.nRanks > 1;
     return 0;
 }
 
@@ -521,8 +639,6 @@ DL_EXPORT int dl_engine_set_trace_all(void *h, int allCtas) {
 
 DL_EXPORT int dl_engine_mega_active(void *h) { return ((Engine *)h)->lastDecodeMega ? 1 : 0; }
 
-DL_EXPORT uint32_t dl_engine_num_sms(void *h) { return ((Engine *)h)->cfg.numSms; }
-
 DL_EXPORT int dl_engine_forward(void *h, int nb, int logitsMode, int greedyAdvance, cudaStream_t stream) {
     return dl::engineForward(*(Engine *)h, nb, logitsMode, greedyAdvance != 0, stream);
 }
@@ -538,12 +654,12 @@ DL_EXPORT int dl_engine_forward_part(void *h, int nb, uint32_t layer, int part, 
     const dl::EngineConfig &c = e.cfg;
     const uint32_t qDim = c.nHeads * c.headDim, kvDim = c.nKvHeads * c.headDim, qkvDim = qDim + 2 * kvDim;
     if (nb < 1 || (uint32_t)nb > c.maxBatch || (nb & (nb - 1))) return -10;
-    if (part == 0) return dl::launchEmbedding(embTable(e), e.g.tokens, e.g.x, c.dim, c.dim, e.g.vocabFull, nb, stream);
+    if (part == 0) return dl::launchEmbedding(embTable(e), e.b.tokens, e.b.x, c.dim, c.dim, c.vocabFull, nb, stream);
     if (part == 3 || part == 4) {
         dl::GemvArgs a{};
         a.qs = (const uint32_t *)e.g.wclsQs; a.scales = (const __half *)e.g.wclsSc; a.d = c.vocab; a.n = c.dim;
-        a.normW = e.g.finalNorm; a.eps = c.eps; a.inStride = c.dim; a.outStride = c.vocab; a.out = e.g.logits;
-        a.in = part == 3 ? e.g.x + (size_t)(nb - 1) * c.dim : e.g.x;
+        a.normW = e.g.finalNorm; a.eps = c.eps; a.inStride = c.dim; a.outStride = c.vocab; a.out = e.b.logits;
+        a.in = part == 3 ? e.b.x + (size_t)(nb - 1) * c.dim : e.b.x;
         return dl::gemvSel(e, dl::PRO_RMSNORM_, dl::EPI_STORE_, part == 3 ? 1 : nb, a, c.numSms, stream, false);
     }
     if (layer >= c.nLayers) return -1;
@@ -551,21 +667,21 @@ DL_EXPORT int dl_engine_forward_part(void *h, int nb, uint32_t layer, int part, 
     dl::GemvArgs a{};
     if (part == 1) {
         a.qs = (const uint32_t *)L.qkvQs; a.scales = (const __half *)L.qkvSc; a.d = qkvDim; a.n = c.dim;
-        a.in = e.g.x; a.inStride = c.dim; a.normW = L.norm0; a.eps = c.eps; a.out = e.g.qkv; a.outStride = qkvDim;
+        a.in = e.b.x; a.inStride = c.dim; a.normW = L.norm0; a.eps = c.eps; a.out = e.b.qkv; a.outStride = qkvDim;
         DL_TRY(dl::gemvSel(e, dl::PRO_RMSNORM_, dl::EPI_STORE_, nb, a, c.numSms, stream, false));
         dl::RopeKvArgs r{};
-        r.qkv = e.g.qkv; r.qkvStride = qkvDim; r.pos = e.g.pos; r.rope = e.g.rope; r.qNorm = L.qNorm; r.kNorm = L.kNorm;
+        r.qkv = e.b.qkv; r.qkvStride = qkvDim; r.pos = e.b.pos; r.rope = e.g.rope; r.qNorm = L.qNorm; r.kNorm = L.kNorm;
         r.eps = c.eps; r.nHeads = c.nHeads; r.nKvHeads = c.nKvHeads; r.headDim = c.headDim; r.seqLen = c.seqLen;
-        r.kCache = (__nv_bfloat16 *)L.kCache; r.vCache = (__nv_bfloat16 *)L.vCache;
+        r.kCache = (__nv_bfloat16 *)e.kCache[layer]; r.vCache = (__nv_bfloat16 *)e.vCache[layer];
         DL_TRY(dl::launchRopeKv(r, nb, stream, false));
         dl::AttnArgs t{};
-        t.qkv = e.g.qkv; t.qkvStride = qkvDim; t.pos = e.g.pos; t.kCache = r.kCache; t.vCache = r.vCache;
+        t.qkv = e.b.qkv; t.qkvStride = qkvDim; t.pos = e.b.pos; t.kCache = r.kCache; t.vCache = r.vCache;
         t.nHeads = c.nHeads; t.nKvHeads = c.nKvHeads; t.headDim = c.headDim; t.seqLen = c.seqLen; t.nSplits = c.nSplits;
-        t.partial = e.g.attnPartial; t.counters = e.g.attnCounters; t.out = e.g.z; t.outStride = qDim;
+        t.partial = e.b.attnPartial; t.counters = e.b.attnCounters; t.out = e.b.z; t.outStride = qDim;
         DL_TRY(dl::launchAttnDecode(t, nb, stream, false));
         a = dl::GemvArgs{};
         a.qs = (const uint32_t *)L.woQs; a.scales = (const __half *)L.woSc; a.d = c.dim; a.n = qDim;
-        a.in = e.g.z; a.inStride = qDim; a.out = ybuf; a.outStride = c.dim;
+        a.in = e.b.z; a.inStride = qDim; a.out = ybuf; a.outStride = c.dim;
         return dl::gemvSel(e, dl::PRO_PLAIN_, dl::EPI_STORE_, nb, a, c.numSms, stream, false);
     }
     if (part == 2 && c.nExperts > 0) {
@@ -575,11 +691,11 @@ DL_EXPORT int dl_engine_forward_part(void *h, int nb, uint32_t layer, int part, 
     }
     if (part == 2) {
         a.qs = (const uint32_t *)L.w13Qs; a.scales = (const __half *)L.w13Sc; a.d = 2 * c.ffDim; a.n = c.dim;
-        a.in = e.g.x; a.inStride = c.dim; a.normW = L.norm1; a.eps = c.eps; a.out = e.g.h; a.outStride = c.ffDim;
+        a.in = e.b.x; a.inStride = c.dim; a.normW = L.norm1; a.eps = c.eps; a.out = e.b.h; a.outStride = c.ffDim;
         DL_TRY(dl::gemvSel(e, dl::PRO_RMSNORM_, dl::EPI_SWIGLU_, nb, a, c.numSms, stream, false));
         a = dl::GemvArgs{};
         a.qs = (const uint32_t *)L.w2Qs; a.scales = (const __half *)L.w2Sc; a.d = c.dim; a.n = c.ffDim;
-        a.in = e.g.h; a.inStride = c.ffDim; a.out = ybuf; a.outStride = c.dim;
+        a.in = e.b.h; a.inStride = c.ffDim; a.out = ybuf; a.outStride = c.dim;
         return dl::gemvSel(e, dl::PRO_PLAIN_, dl::EPI_STORE_, nb, a, c.numSms, stream, false);
     }
     return -2;

@@ -11,15 +11,17 @@ constexpr int kApiMaxRanks = 8;
 struct EngineConfig {   // mirrored by ctypes in distributed_llama_b200/ops/cuda_lib.py
     uint32_t dim, nLayers, nHeads, nKvHeads, headDim, ffDim, vocab, seqLen;   // per-rank (sliced) head/ff/vocab counts
     uint32_t nExperts, nActiveExperts;
-    uint32_t maxBatch;       // tokens per forward on the GEMV path
-    uint32_t nSplits;        // attention KV splits
+    uint32_t maxBatch;       // tokens per forward on the GEMV path (mixture of experts: always 1)
+    uint32_t nSplits;        // attention KV splits (0: max(1, min(32, 2 * numSms / nHeads)))
     uint32_t rank, nRanks;
-    uint32_t numSms;
+    uint32_t numSms;         // 0: the current device's SM count
     float eps;
     uint32_t usePdl;
     uint32_t moeFirstExpert, moeNumLocal;   // experts held by this rank (expert parallelism); TP mode: 0, nExperts
     uint32_t wType;          // matrix storage: 0 = q40 device layout, 1 = dense f32, 2 = dense f16 (gemv_dense.cu)
     uint32_t hiddenAct;      // gate activation: 0 = SiLU, 1 = GELU (tanh form) — the `.m` header's hidden_act
+    uint32_t vocabFull;      // rows of the whole embedding table
+    uint32_t maxPrefill;     // tokens per chunk on the tensor-core prefill path (at most 256)
 };
 
 struct LayerPtrs {
@@ -29,7 +31,6 @@ struct LayerPtrs {
     const void *w2Qs, *w2Sc;     // [dim][ff];                          MoE: [nExperts][dim][ff]
     const float *norm0, *norm1, *qNorm, *kNorm;
     const float *moeGate;        // [nExperts][dim] f32
-    void *kCache, *vCache;       // bf16 [nKvHeads][seqLen][hd]
 };
 
 struct GlobalPtrs {
@@ -39,49 +40,33 @@ struct GlobalPtrs {
     const float *finalNorm;
     const void *wclsQs, *wclsSc; // [vocab][dim]
     const float *rope;           // [seqLen][hd/2][2]
-    uint32_t vocabFull;
-    // activations / state
-    int *tokens, *pos;           // [maxBatch]
-    float *x, *qkv, *z, *h, *logits;   // [maxBatch][dim | qkvDim | qDim | ff | vocab]
-    float *attnPartial;          // [maxBatch][nHeads][nSplits][hd+2]
-    unsigned int *attnCounters;  // [maxBatch][nHeads]
-    int *history;                // [seqLen] generated token per position (device-side log), may be null
-    // MoE scratch
-    int *expertIdx;              // [maxBatch][nActive]
-    float *expertWeight;         // [maxBatch][nActive]
-    float *routerLogits;         // [maxBatch][nExperts]
-    unsigned int *routerCounter; // [maxBatch]
-    float *moeScratch;           // [nActive][dim]
-    unsigned int *moeCounters;   // [256]
-    // prefill (tensor-core GEMM path) buffers, maxPrefill tokens
-    uint32_t maxPrefill;
-    int *pTokens, *pPos;         // [maxPrefill]
-    float *px, *pqkv;            // [maxPrefill][dim | qkvDim] f32
-    void *pxn, *pzb, *phb;       // bf16 [maxPrefill][dim | qDim | ff]
-    float *pAttnPartial;         // [maxPrefill][nHeads][hd+2]
-    unsigned int *pAttnCounters; // [maxPrefill][nHeads]
-    // fused arg-max scratch
-    float *argVal;               // [numSms]
-    int *argIdx;                 // [numSms]
-    unsigned int *argCounter;    // [1]
+};
+
+// Device memory owned by the engine (allocated and zeroed by dl_engine_create) that a front end reads or writes.
+struct EngineBuffers {
+    int *tokens, *pos;           // [maxBatch] tokens and positions of a forward; decoding advances tokens[0] / pos[0] on the device
+    int *history;                // [seqLen + 1] generated token per position
+    float *logits;               // [maxBatch][vocab]
+    float *x;                    // [maxBatch][dim] residual stream
+    int *pTokens, *pPos;         // [maxPrefill] tokens and positions of a prefill chunk
+    void *const *kCache, *const *vCache;   // [nLayers] (host arrays) bf16 [nKvHeads][seqLen][hd]
 };
 
 struct CommPtrs {   // mirrored by ctypes
-    uint32_t nRanks, rank, maxCtas, slotStride;
-    void *arena[kApiMaxRanks];          // every rank's symmetric arena mapped into this process
+    void *arena[kApiMaxRanks];          // every rank's symmetric arena (dl_engine_arena_bytes each) mapped into this process
     void *mcArena;                      // NVLS multicast mapping of the arena (null: none)
-    uint64_t slotsOff, flagsOff, candValOff, gatherOff;   // LL all-reduce slots, logits-gather arrival counters, arg-max candidates, gathered logits
-    uint64_t prefillSlotsOff;        // LL slots for the prefill GEMM all-reduce: [2][nRanks][maxPrefill * dim]
-    uint32_t prefillSlotStride;
 };
 
 }  // namespace dl
 
 extern "C" {
-void *dl_engine_create(const dl::EngineConfig *cfg);
+void *dl_engine_create(const dl::EngineConfig *cfg);   // allocates on the current device; null on failure
 void dl_engine_destroy(void *h);
 int dl_engine_set_layer(void *h, uint32_t layer, const dl::LayerPtrs *p);
 int dl_engine_set_globals(void *h, const dl::GlobalPtrs *p);
+int dl_engine_get_config(void *h, dl::EngineConfig *cfg);   // the values the engine uses (defaults and limits applied)
+int dl_engine_buffers(void *h, dl::EngineBuffers *b);
+size_t dl_engine_arena_bytes(const dl::EngineConfig *cfg);   // peer arena per rank for tensor parallelism; no CUDA calls
 int dl_engine_set_comm(void *h, const dl::CommPtrs *p);
 int dl_engine_enable_mega(void *h, int enable);
 int dl_engine_set_vocab_limit(void *h, uint32_t limit);   // greedy arg-max never returns ids >= limit (tokenizer vocabulary size)
@@ -92,7 +77,6 @@ int dl_engine_sampler_seed(void *h, unsigned long long seed);
 int dl_engine_sample(void *h, float temperature, float topp, cudaStream_t stream);   // after a forward with logitsMode 1
 int dl_engine_set_trace(void *h, uint64_t *buf, uint32_t capLaunches);
 int dl_engine_set_trace_all(void *h, int allCtas);
-uint32_t dl_engine_num_sms(void *h);
 int dl_engine_forward(void *h, int nb, int logitsMode, int greedyAdvance, cudaStream_t stream);
 int dl_engine_forward_part(void *h, int nb, uint32_t layer, int part, float *ybuf, cudaStream_t stream);
 int dl_engine_prefill(void *h, uint32_t T, uint32_t p0, int wantLogits, cudaStream_t stream);   // T tokens staged in pTokens/pPos at positions p0 .. p0 + T - 1

@@ -23,6 +23,7 @@ import torch
 from .. import host
 from ..formats.model_file import ModelFile
 from ..formats import quants
+from ..ops import cuda_lib as cl
 from ..ops.q40 import DeviceDense, DeviceQ40, repack_q40
 from .config import ROPE_FALCON
 
@@ -155,12 +156,6 @@ def _load_dense(mf: ModelFile, up: "_Uploader", rank, n_ranks, kv_rank, kv_ranks
     return W
 
 
-class _RawCuda:
-    """Wraps a raw device pointer (peer-mapped VMM memory) as a CUDA array so torch can view it."""
-    def __init__(self, ptr: int, n_floats: int):
-        self.__cuda_array_interface__ = {"shape": (n_floats,), "typestr": "<f4", "data": (ptr, False), "version": 2}
-
-
 def _sharded_embedding(mf: ModelFile, up: "_Uploader", rank: int, n_ranks: int, device, comm):
     """Uploads only this rank's vocabulary rows of the f32 embedding into peer-mapped memory; returns (local tensor, pointers of all
     shards, rows per shard) or None when no symmetric allocation is available (the table is then replicated)."""
@@ -174,7 +169,7 @@ def _sharded_embedding(mf: ModelFile, up: "_Uploader", rank: int, n_ranks: int, 
     ptrs = comm.alloc_shared(rows * h.dim * 4)
     if ptrs is None:
         return None
-    local = torch.as_tensor(_RawCuda(ptrs[rank], rows * h.dim), device=device).view(rows, h.dim)
+    local = cl.device_view(ptrs[rank], (rows, h.dim), torch.float32, device=device)
     e = mf.entry("embedding")
     src = mf.data[e.offset + rank * rows * h.dim * 4: e.offset + (rank + 1) * rows * h.dim * 4]
     with warnings.catch_warnings():

@@ -18,28 +18,40 @@ u32, u64, i32, f32, vp = C.c_uint32, C.c_uint64, C.c_int, C.c_float, C.c_void_p
 class EngineConfig(C.Structure):
     _fields_ = [(n, u32) for n in ("dim", "nLayers", "nHeads", "nKvHeads", "headDim", "ffDim", "vocab", "seqLen",
                                    "nExperts", "nActiveExperts", "maxBatch", "nSplits", "rank", "nRanks", "numSms")] + \
-               [("eps", f32), ("usePdl", u32), ("moeFirstExpert", u32), ("moeNumLocal", u32), ("wType", u32), ("hiddenAct", u32)]
+               [("eps", f32), ("usePdl", u32), ("moeFirstExpert", u32), ("moeNumLocal", u32), ("wType", u32), ("hiddenAct", u32),
+                ("vocabFull", u32), ("maxPrefill", u32)]
 
 
 class LayerPtrs(C.Structure):
     _fields_ = [(n, vp) for n in ("qkvQs", "qkvSc", "woQs", "woSc", "w13Qs", "w13Sc", "w2Qs", "w2Sc",
-                                  "norm0", "norm1", "qNorm", "kNorm", "moeGate", "kCache", "vCache")]
+                                  "norm0", "norm1", "qNorm", "kNorm", "moeGate")]
 
 
 class GlobalPtrs(C.Structure):
-    _fields_ = [("embedding", vp), ("embeddingPeers", vp * 8), ("embRowsPerRank", u32), ("finalNorm", vp), ("wclsQs", vp), ("wclsSc", vp), ("rope", vp), ("vocabFull", u32),
-                ("tokens", vp), ("pos", vp), ("x", vp), ("qkv", vp), ("z", vp), ("h", vp), ("logits", vp),
-                ("attnPartial", vp), ("attnCounters", vp), ("history", vp), ("expertIdx", vp), ("expertWeight", vp),
-                ("routerLogits", vp), ("routerCounter", vp), ("moeScratch", vp), ("moeCounters", vp),
-                ("maxPrefill", u32), ("pTokens", vp), ("pPos", vp), ("px", vp), ("pqkv", vp), ("pxn", vp), ("pzb", vp), ("phb", vp),
-                ("pAttnPartial", vp), ("pAttnCounters", vp),
-                ("argVal", vp), ("argIdx", vp), ("argCounter", vp)]
+    _fields_ = [("embedding", vp), ("embeddingPeers", vp * 8), ("embRowsPerRank", u32), ("finalNorm", vp), ("wclsQs", vp), ("wclsSc", vp),
+                ("rope", vp)]
+
+
+class EngineBuffers(C.Structure):
+    _fields_ = [(n, vp) for n in ("tokens", "pos", "history", "logits", "x", "pTokens", "pPos")] + \
+               [("kCache", C.POINTER(vp)), ("vCache", C.POINTER(vp))]
 
 
 class CommPtrs(C.Structure):
-    _fields_ = [("nRanks", u32), ("rank", u32), ("maxCtas", u32), ("slotStride", u32), ("arena", vp * 8), ("mcArena", vp),
-                ("slotsOff", u64), ("flagsOff", u64), ("candValOff", u64),
-                ("gatherOff", u64), ("prefillSlotsOff", u64), ("prefillSlotStride", u32)]
+    _fields_ = [("arena", vp * 8), ("mcArena", vp)]
+
+
+class _DeviceArray:
+    def __init__(self, ptr: int, shape, typestr: str, owner):
+        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (ptr, False), "version": 2}
+        self.owner = owner
+
+
+def device_view(ptr: int, shape, dtype, owner=None, device=None):
+    """A torch tensor over device memory torch did not allocate. `owner` stays alive as long as the tensor or any view of it."""
+    import torch
+    typestr = {torch.float32: "<f4", torch.int32: "<i4", torch.bfloat16: "<i2"}[dtype]   # the interface has no bf16 type
+    return torch.as_tensor(_DeviceArray(ptr, shape, typestr, owner), device=device).view(dtype)
 
 
 def lib() -> C.CDLL:
@@ -70,6 +82,12 @@ def lib() -> C.CDLL:
     L.dl_engine_set_layer.restype = i32
     L.dl_engine_set_globals.argtypes = [vp, C.POINTER(GlobalPtrs)]
     L.dl_engine_set_globals.restype = i32
+    L.dl_engine_get_config.argtypes = [vp, C.POINTER(EngineConfig)]
+    L.dl_engine_get_config.restype = i32
+    L.dl_engine_buffers.argtypes = [vp, C.POINTER(EngineBuffers)]
+    L.dl_engine_buffers.restype = i32
+    L.dl_engine_arena_bytes.argtypes = [C.POINTER(EngineConfig)]
+    L.dl_engine_arena_bytes.restype = C.c_size_t
     L.dl_engine_enable_mega.argtypes = [vp, i32]
     L.dl_engine_enable_mega.restype = i32
     L.dl_engine_set_vocab_limit.argtypes = [vp, u32]
@@ -112,8 +130,6 @@ def lib() -> C.CDLL:
     L.dl_engine_aborted.restype = i32
     L.dl_engine_set_trace_all.argtypes = [vp, i32]
     L.dl_engine_set_trace_all.restype = i32
-    L.dl_engine_num_sms.argtypes = [vp]
-    L.dl_engine_num_sms.restype = u32
     L.dl_engine_forward.argtypes = [vp, i32, i32, i32, vp]
     L.dl_engine_forward.restype = i32
     L.dl_engine_forward_part.argtypes = [vp, i32, u32, i32, vp, vp]
@@ -129,7 +145,6 @@ def lib() -> C.CDLL:
 
 
 _ERRORS = {
-    -12: "prompt chunk larger than the prefill all-reduce slots of the peer arena",
     -30: "tensor-parallel slice too narrow for the fused all-reduce GEMV: the per-rank K of WO / W2 (heads/N * headDim, ffDim/N) "
          "must be a multiple of 128 — use fewer ranks, or DL_COLLECTIVES=nccl",
     -31: "mixture-of-experts up-projection shape not covered by the TMA GEMV",

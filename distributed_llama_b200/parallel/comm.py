@@ -7,39 +7,12 @@ root/worker TCP mesh bootstrap and the per-segment sync steps. Here rank 0 is th
 from __future__ import annotations
 
 import ctypes as C
-from dataclasses import dataclass
 from typing import List
 
 import torch
 import torch.distributed as dist
 
 from ..ops import cuda_lib as cl
-
-MAX_CTAS = 256
-
-
-@dataclass
-class ArenaLayout:
-    slots_off: int
-    flags_off: int
-    cand_val_off: int
-    gather_off: int
-    prefill_slots_off: int
-    prefill_slot_stride: int
-    total: int
-
-
-def arena_layout(n_ranks: int, max_batch: int, dim: int, vocab_full: int, max_prefill: int = 0) -> ArenaLayout:
-    def align(x):
-        return (x + 255) // 256 * 256
-    off = 0
-    slots = off; off = align(off + 2 * n_ranks * max_batch * dim * 8)   # LL words: (f32 payload, flag)
-    flags = off; off = align(off + 2 * n_ranks * MAX_CTAS * 4)            # logits-gather arrival counters (sampler.cu)
-    cv = off; off = align(off + 8 * 8)                                   # arg-max candidates, one LL word per rank
-    gather = off; off = align(off + max_batch * vocab_full * 4)
-    pslots = off; off = align(off + 2 * n_ranks * max_prefill * dim * 8)
-    return ArenaLayout(slots, flags, cv, gather, pslots, max_prefill * dim, off)
-
 
 class Communicator:
     """Wraps the default process group. `alloc_arena` creates the symmetric buffer and maps every peer's copy."""
@@ -54,7 +27,6 @@ class Communicator:
         self.arena_ptrs: List[int] = []
         self.mc_ptr: int = 0             # NVLS multicast mapping of the arena (0: not available, kernels use unicast peer stores)
         self.arena_kind = "none"         # "vmm" (cuMem* + multicast) or "ipc" (cudaMalloc + CUDA IPC)
-        self.layout: ArenaLayout | None = None
         self._local = None
         self._vmm = None
         # Peer-memory (CUDA IPC over NVLink) collectives need every rank on one host; otherwise the engine falls back to NCCL.
@@ -69,14 +41,13 @@ class Communicator:
 
     _arena_seq = 0
 
-    def alloc_arena(self, layout: ArenaLayout) -> None:
-        """Creates the symmetric arena. Preferred: CUDA VMM allocation shared through POSIX descriptors with an NVLS multicast
-        mapping (csrc/cuda/comm_vmm.cu); fallback: cudaMalloc + CUDA IPC handles (no multicast)."""
+    def alloc_arena(self, nbytes: int) -> None:
+        """Creates the symmetric arena of `nbytes` per rank. Preferred: CUDA VMM allocation shared through POSIX descriptors with
+        an NVLS multicast mapping (csrc/cuda/comm_vmm.cu); fallback: cudaMalloc + CUDA IPC handles (no multicast)."""
         import os
-        self.layout = layout
-        if os.environ.get("DL_NO_VMM") is None and self.single_node and self._alloc_vmm(layout):
+        if os.environ.get("DL_NO_VMM") is None and self.single_node and self._alloc_vmm(nbytes):
             return
-        self._alloc_ipc(layout)
+        self._alloc_ipc(nbytes)
 
     def alloc_shared(self, nbytes: int):
         """A second symmetric allocation (no multicast mapping): returns the list of per-rank device pointers, or None when the VMM
@@ -91,8 +62,8 @@ class Communicator:
         self._shared_handles = getattr(self, "_shared_handles", []) + [h]
         return ptrs
 
-    def _alloc_vmm(self, layout: ArenaLayout) -> bool:
-        res = self._vmm_bootstrap(layout.total, want_mc=0 if __import__("os").environ.get("DL_NO_MULTICAST") is not None else 1)
+    def _alloc_vmm(self, nbytes: int) -> bool:
+        res = self._vmm_bootstrap(nbytes, want_mc=0 if __import__("os").environ.get("DL_NO_MULTICAST") is not None else 1)
         if res is None:
             return False
         self._vmm, self.arena_ptrs, self.mc_ptr = res
@@ -136,9 +107,9 @@ class Communicator:
         dist.barrier()
         return h, ptrs, mc_ptr
 
-    def _alloc_ipc(self, layout: ArenaLayout) -> None:
+    def _alloc_ipc(self, nbytes: int) -> None:
         ptr = C.c_void_p()
-        cl.check(self._lib.dl_comm_alloc(layout.total, C.byref(ptr)), "comm_alloc")
+        cl.check(self._lib.dl_comm_alloc(nbytes, C.byref(ptr)), "comm_alloc")
         self._local = ptr.value
         handle = (C.c_ubyte * 64)()
         cl.check(self._lib.dl_comm_ipc_handle(ptr, handle), "comm_ipc_handle")
@@ -157,15 +128,6 @@ class Communicator:
         self.mc_ptr = 0
         self.arena_kind = "ipc"
         dist.barrier()
-
-    def comm_ptrs(self, slot_stride: int) -> cl.CommPtrs:
-        L = self.layout
-        arr = (C.c_void_p * 8)(*([C.c_void_p(p) for p in self.arena_ptrs] + [None] * (8 - len(self.arena_ptrs))))
-        return cl.CommPtrs(nRanks=self.world_size, rank=self.rank, maxCtas=MAX_CTAS, slotStride=slot_stride, arena=arr,
-                           mcArena=C.c_void_p(self.mc_ptr) if self.mc_ptr else None,
-                           slotsOff=L.slots_off, flagsOff=L.flags_off, candValOff=L.cand_val_off,
-                           gatherOff=L.gather_off, prefillSlotsOff=L.prefill_slots_off,
-                           prefillSlotStride=L.prefill_slot_stride)
 
     # ---- baseline collectives (NCCL) ----
     def all_reduce(self, t: torch.Tensor) -> torch.Tensor:

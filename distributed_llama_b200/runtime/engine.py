@@ -1,8 +1,8 @@
 """Python handle of the native per-rank engine (csrc/cuda/engine.cu).
 
-Owns the device tensors (weights, KV cache, activation buffers), hands their pointers to the C++ engine and exposes
-the three calls the apps need: `prefill(tokens, pos)`, `step(token, pos)` -> logits, and the device-resident greedy
-decode loop `decode_greedy(n)` that replays the captured CUDA graph.
+Hands the weight pointers to the C++ engine, which owns the KV cache and activation buffers (`tokens`, `logits`, `k_cache`,
+... are torch views of its memory), and exposes the three calls the apps need: `prefill(tokens, pos)`, `step(token, pos)`
+-> logits, and the device-resident greedy decode loop `decode_greedy(n)` that replays the captured CUDA graph.
 Plays the role of the reference's RootLlmInference (src/app.cpp:168-208): setBatchSize/setPosition/setToken/forward.
 """
 from __future__ import annotations
@@ -22,6 +22,27 @@ def _p(t: Optional[torch.Tensor]):
     return t.data_ptr() if t is not None else None
 
 
+def _ptrs8(ptrs):
+    return (C.c_void_p * 8)(*ptrs, *([None] * (8 - len(ptrs))))
+
+
+class _Handle:
+    """Owns the native engine. The Engine and every view of engine memory hold it, so the memory outlives them all."""
+
+    def __init__(self, lib, cfg):
+        self.lib = lib
+        self.h = lib.dl_engine_create(C.byref(cfg))
+        if not self.h:
+            raise RuntimeError("dl_engine_create failed: cannot allocate the engine's device memory")
+
+    def __del__(self):
+        try:
+            if getattr(self, "h", None):
+                self.lib.dl_engine_destroy(self.h)
+        except Exception:
+            pass
+
+
 class Engine:
     def __init__(self, weights: DeviceWeights, max_batch: int = 8, n_splits: int = 0, use_pdl: bool = True,
                  seq_len: Optional[int] = None, comm=None, max_prefill: int = 192, collectives: str = "auto"):
@@ -30,8 +51,6 @@ class Engine:
         dev = w.embedding.device
         self.device = dev
         self.seq_len = seq_len or h.seq_len
-        if h.n_experts > 0:
-            max_batch = 1          # the MoE kernels route one token per launch
         self.dense = getattr(w, "weight_kind", 0) != 0
         if self.dense:
             # f32 activations of all tokens of a launch are staged in shared memory (gemv_dense.cu)
@@ -41,77 +60,40 @@ class Engine:
                 raise ValueError("matrix rows too wide for the dense-weight kernels on one GPU; use more ranks")
             while max_batch > cap:
                 max_batch //= 2
-        self.max_batch = max_batch
-        props = torch.cuda.get_device_properties(dev)
-        self.num_sms = props.multi_processor_count
-        if n_splits <= 0:
-            n_splits = max(1, min(32, (2 * self.num_sms) // max(1, w.n_heads)))
-        self.n_splits = n_splits
-        hd = h.head_dim
-        q_dim, kv_dim = w.n_heads * hd, w.n_kv_heads * hd
-        self.qkv_dim = q_dim + 2 * kv_dim
-        f32 = dict(dtype=torch.float32, device=dev)
-        self.tokens = torch.zeros(max_batch, dtype=torch.int32, device=dev)
-        self.pos = torch.zeros(max_batch, dtype=torch.int32, device=dev)
-        self.x = torch.zeros(max_batch, h.dim, **f32)
-        self.qkv = torch.zeros(max_batch, self.qkv_dim, **f32)
-        self.z = torch.zeros(max_batch, q_dim, **f32)
-        self.h = torch.zeros(max(max_batch, h.n_active_experts, 1), w.ff_dim, **f32)
-        self.router_logits = torch.zeros(max_batch * max(1, h.n_experts), **f32)
-        self.router_counter = torch.zeros(max_batch, dtype=torch.int32, device=dev)
-        self.moe_scratch = torch.zeros(max(1, h.n_active_experts) * h.dim, **f32)
-        self.moe_counters = torch.zeros(256, dtype=torch.int32, device=dev)
-        self.logits = torch.zeros(max_batch, w.vocab, **f32)
-        self.attn_partial = torch.zeros(max_batch * w.n_heads * n_splits * (hd + 2), **f32)
-        self.attn_counters = torch.zeros(max_batch * w.n_heads, dtype=torch.int32, device=dev)
-        self.history = torch.zeros(self.seq_len + 1, dtype=torch.int32, device=dev)
-        self.k_cache = [torch.zeros(w.n_kv_heads, self.seq_len, hd, dtype=torch.bfloat16, device=dev) for _ in range(h.n_layers)]
-        self.v_cache = [torch.zeros(w.n_kv_heads, self.seq_len, hd, dtype=torch.bfloat16, device=dev) for _ in range(h.n_layers)]
-        self.expert_idx = torch.zeros(max_batch * max(1, h.n_active_experts), dtype=torch.int32, device=dev)
-        self.expert_weight = torch.zeros(max_batch * max(1, h.n_active_experts), **f32)
-        self.max_prefill = mp = min(max_prefill, 256)
-        bf16 = dict(dtype=torch.bfloat16, device=dev)
-        self.p_tokens = torch.zeros(mp, dtype=torch.int32, device=dev)
-        self.p_pos = torch.zeros(mp, dtype=torch.int32, device=dev)
-        self.p_x = torch.zeros(mp, h.dim, **f32)
-        self.p_qkv = torch.zeros(mp, max(self.qkv_dim, h.dim), **f32)   # also the [T][dim] partial of the TP WO / W2 GEMMs
-        self.p_xn = torch.zeros(mp, h.dim, **bf16)
-        self.p_zb = torch.zeros(mp, q_dim, **bf16)
-        self.p_hb = torch.zeros(mp, w.ff_dim, **bf16)
-        self.p_attn_partial = torch.zeros(mp * w.n_heads * (hd + 2), **f32)
-        self.p_attn_counters = torch.zeros(mp * w.n_heads, dtype=torch.int32, device=dev)
-        self.arg_val = torch.zeros(256, **f32)
-        self.arg_idx = torch.zeros(256, dtype=torch.int32, device=dev)
-        self.arg_counter = torch.zeros(4, dtype=torch.int32, device=dev)
-
-        cfg = cl.EngineConfig(dim=h.dim, nLayers=h.n_layers, nHeads=w.n_heads, nKvHeads=w.n_kv_heads, headDim=hd,
+        cfg = cl.EngineConfig(dim=h.dim, nLayers=h.n_layers, nHeads=w.n_heads, nKvHeads=w.n_kv_heads, headDim=h.head_dim,
                               ffDim=w.ff_dim, vocab=w.vocab, seqLen=self.seq_len, nExperts=h.n_experts,
-                              nActiveExperts=h.n_active_experts, maxBatch=max_batch, nSplits=n_splits, rank=w.rank,
-                              nRanks=w.n_ranks, numSms=self.num_sms, eps=h.norm_epsilon, usePdl=1 if use_pdl else 0,
+                              nActiveExperts=h.n_active_experts, maxBatch=max_batch, nSplits=max(0, n_splits), rank=w.rank,
+                              nRanks=w.n_ranks, numSms=0, eps=h.norm_epsilon, usePdl=1 if use_pdl else 0,
                               moeFirstExpert=w.first_expert, moeNumLocal=w.n_local_experts,
                               wType=getattr(w, "weight_kind", 0),
-                              hiddenAct=1 if int(h.hidden_act) == 0 else 0)   # header: ACT_GELU = 0, ACT_SILU = 1
+                              hiddenAct=1 if int(h.hidden_act) == 0 else 0,   # header: ACT_GELU = 0, ACT_SILU = 1
+                              vocabFull=h.vocab_size, maxPrefill=max_prefill)
         self._lib = cl.lib()
-        self._h = self._lib.dl_engine_create(C.byref(cfg))
+        with torch.cuda.device(dev):
+            owner = _Handle(self._lib, cfg)
+        self._owner, self._h = owner, owner.h
+        cl.check(self._lib.dl_engine_get_config(self._h, C.byref(cfg)), "engine_get_config")
+        mb, mp = cfg.maxBatch, cfg.maxPrefill   # the engine's limits applied
+        self.max_batch, self.max_prefill, self.num_sms = mb, mp, cfg.numSms
         for l, L in enumerate(w.layers):
             lp = cl.LayerPtrs(qkvQs=_p(L.qkv.qs), qkvSc=_p(L.qkv.scales), woQs=_p(L.wo.qs), woSc=_p(L.wo.scales),
                               w13Qs=_p(L.w13.qs), w13Sc=_p(L.w13.scales), w2Qs=_p(L.w2.qs), w2Sc=_p(L.w2.scales),
-                              norm0=_p(L.norm0), norm1=_p(L.norm1), qNorm=_p(L.q_norm), kNorm=_p(L.k_norm),
-                              moeGate=_p(L.moe_gate), kCache=_p(self.k_cache[l]), vCache=_p(self.v_cache[l]))
+                              norm0=_p(L.norm0), norm1=_p(L.norm1), qNorm=_p(L.q_norm), kNorm=_p(L.k_norm), moeGate=_p(L.moe_gate))
             cl.check(self._lib.dl_engine_set_layer(self._h, l, C.byref(lp)), "engine_set_layer")
-        emb_peers = (C.c_void_p * 8)(*([C.c_void_p(p) for p in (w.embedding_ptrs or [])] + [None] * (8 - len(w.embedding_ptrs or []))))
-        gp = cl.GlobalPtrs(embedding=_p(w.embedding), embeddingPeers=emb_peers, embRowsPerRank=w.embedding_rows or 0, finalNorm=_p(w.final_norm), wclsQs=_p(w.wcls.qs),
-                           wclsSc=_p(w.wcls.scales), rope=_p(w.rope), vocabFull=h.vocab_size, tokens=_p(self.tokens),
-                           pos=_p(self.pos), x=_p(self.x), qkv=_p(self.qkv), z=_p(self.z), h=_p(self.h),
-                           logits=_p(self.logits), attnPartial=_p(self.attn_partial), attnCounters=_p(self.attn_counters),
-                           history=_p(self.history), expertIdx=_p(self.expert_idx), expertWeight=_p(self.expert_weight),
-                           routerLogits=_p(self.router_logits), routerCounter=_p(self.router_counter),
-                           moeScratch=_p(self.moe_scratch), moeCounters=_p(self.moe_counters),
-                           maxPrefill=mp, pTokens=_p(self.p_tokens), pPos=_p(self.p_pos), px=_p(self.p_x), pqkv=_p(self.p_qkv),
-                           pxn=_p(self.p_xn), pzb=_p(self.p_zb), phb=_p(self.p_hb), pAttnPartial=_p(self.p_attn_partial),
-                           pAttnCounters=_p(self.p_attn_counters),
-                           argVal=_p(self.arg_val), argIdx=_p(self.arg_idx), argCounter=_p(self.arg_counter))
+        gp = cl.GlobalPtrs(embedding=_p(w.embedding), embeddingPeers=_ptrs8(w.embedding_ptrs or []), embRowsPerRank=w.embedding_rows or 0,
+                           finalNorm=_p(w.final_norm), wclsQs=_p(w.wcls.qs), wclsSc=_p(w.wcls.scales), rope=_p(w.rope))
         cl.check(self._lib.dl_engine_set_globals(self._h, C.byref(gp)), "engine_set_globals")
+        b = cl.EngineBuffers()
+        cl.check(self._lib.dl_engine_buffers(self._h, C.byref(b)), "engine_buffers")
+
+        def view(ptr, shape, dtype=torch.int32):
+            return cl.device_view(ptr, shape, dtype, owner, dev)
+        self.tokens, self.pos, self.history = view(b.tokens, (mb,)), view(b.pos, (mb,)), view(b.history, (self.seq_len + 1,))
+        self.logits, self.x = view(b.logits, (mb, w.vocab), torch.float32), view(b.x, (mb, h.dim), torch.float32)
+        self.p_tokens, self.p_pos = view(b.pTokens, (mp,)), view(b.pPos, (mp,))
+        kv = (w.n_kv_heads, self.seq_len, h.head_dim)
+        self.k_cache = [view(b.kCache[l], kv, torch.bfloat16) for l in range(h.n_layers)]
+        self.v_cache = [view(b.vCache[l], kv, torch.bfloat16) for l in range(h.n_layers)]
         self.comm = comm
         tp = comm is not None and comm.world_size > 1
         # Collectives: "fused" = inside the kernels over NVLink peer memory (ranks of one node, q40 weights);
@@ -121,28 +103,19 @@ class Engine:
                    or not getattr(comm, "single_node", True)):
             self.collectives = "nccl"
         if tp and self.collectives == "fused":
-            from ..parallel.comm import arena_layout
-            comm.alloc_arena(arena_layout(comm.world_size, max_batch, h.dim, h.vocab_size, self.max_prefill))
-            cp = comm.comm_ptrs(max_batch * h.dim)
+            comm.alloc_arena(self._lib.dl_engine_arena_bytes(C.byref(cfg)))
+            cp = cl.CommPtrs(arena=_ptrs8(comm.arena_ptrs), mcArena=comm.mc_ptr or None)
             cl.check(self._lib.dl_engine_set_comm(self._h, C.byref(cp)), "engine_set_comm")
         self._parts = tp and self.collectives == "nccl"
-        self._ybuf = torch.zeros(max_batch, h.dim, **f32)
+        self._ybuf = torch.zeros(mb, h.dim, dtype=torch.float32, device=dev)
         self.use_tc_prefill = not self.dense and not self._parts
         self.mega = False
         if h.n_experts == 0 and not self.dense and not self._parts and os.environ.get("DL_NO_MEGA") is None:
             self.enable_mega(True)     # persistent decode kernel by default; the engine falls back per call if a shape is unsupported
         self.tc_min_tokens = 9          # shorter chunks stay on the GEMV path
         self._graph_ready = False
-        self._stage_tok = torch.zeros(max_batch, dtype=torch.int32).pin_memory()
-        self._stage_pos = torch.zeros(max_batch, dtype=torch.int32).pin_memory()
-
-    def __del__(self):
-        try:
-            if getattr(self, "_h", None):
-                self._lib.dl_engine_destroy(self._h)
-                self._h = None
-        except Exception:
-            pass
+        self._stage_tok = torch.zeros(mb, dtype=torch.int32).pin_memory()
+        self._stage_pos = torch.zeros(mb, dtype=torch.int32).pin_memory()
 
     def set_vocab_limit(self, limit: int):
         """Greedy arg-max on the device never returns ids >= limit (the tokenizer's vocabulary size: embeddings may be padded

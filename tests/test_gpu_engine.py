@@ -77,6 +77,19 @@ def test_tensor_core_prefill_matches_oracle(tmp_models, name):
     assert (lg - lg_b).abs().max().item() < 0.12
 
 
+def test_views_outlive_engine(tmp_models):
+    """`logits` is a view of engine-owned memory: it keeps the engine alive after the Engine object is dropped."""
+    import gc
+    eng = _setup(tmp_models, "tiny-llama31")[1]
+    eng.step(3, 0)
+    logits, want = eng.logits, eng.logits.clone()
+    del eng
+    gc.collect()
+    other = _setup(tmp_models, "tiny-llama31")[1]   # would be handed the freed memory if the view did not hold it
+    torch.cuda.synchronize()
+    assert torch.equal(logits.clone(), want) and other.logits.data_ptr() != logits.data_ptr()
+
+
 @pytest.mark.parametrize("name", ["tiny-llama31", "tiny-qwen3"])
 def test_persistent_decode_kernel(tmp_models, name):
     """The one-launch-per-token megakernel must reproduce the multi-kernel path (logits close, greedy tokens equal)."""

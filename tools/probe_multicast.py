@@ -3,7 +3,6 @@
 Checks, on every rank: unicast peer stores land in every arena; `multimem.red.add` on the multicast mapping is applied to every
 replica; `multimem.ld_reduce` returns the switch-side sum. Prints one PROBE line per rank and `PROBE PASS` / `PROBE FAIL`.
 """
-import ctypes as C
 import os
 import sys
 
@@ -12,7 +11,7 @@ import torch
 import torch.distributed as dist
 
 from distributed_llama_b200.ops import cuda_lib as cl
-from distributed_llama_b200.parallel.comm import ArenaLayout, Communicator
+from distributed_llama_b200.parallel.comm import Communicator
 
 rank, local = int(os.environ["RANK"]), int(os.environ["LOCAL_RANK"])
 torch.cuda.set_device(local)
@@ -21,17 +20,13 @@ comm = Communicator()
 n = 4096
 W = comm.world_size
 total = (4 + W) * n * 4 + 4096
-comm.alloc_arena(ArenaLayout(0, 0, 0, 0, 0, 0, 0, 0, total))
+comm.alloc_arena(total)
 lib = cl.lib()
 print(f"PROBE rank {rank}: arena kind={comm.arena_kind} mc_ptr={'0x%x' % comm.mc_ptr if comm.mc_ptr else 0} "
       f"uc={[hex(p) for p in comm.arena_ptrs]}", flush=True)
 ok = True
 if comm.arena_kind == "vmm":
-    # wrap the local arena as a torch tensor through the CUDA array interface
-    class _Mem:
-        def __init__(self, ptr, nfloats):
-            self.__cuda_array_interface__ = {"shape": (nfloats,), "typestr": "<f4", "data": (ptr, False), "version": 2}
-    arena = torch.as_tensor(_Mem(comm.arena_ptrs[rank], (4 + W) * n), device=f"cuda:{local}")
+    arena = cl.device_view(comm.arena_ptrs[rank], ((4 + W) * n,), torch.float32, device=f"cuda:{local}")
     # region 2+W: every rank writes its own value, later summed by multimem.ld_reduce
     arena[(2 + W) * n:(3 + W) * n] = float(10 * (rank + 1))
     torch.cuda.synchronize()
