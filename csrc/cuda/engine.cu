@@ -39,6 +39,9 @@ struct Buffers {   // working memory of the kernels, allocated and zeroed by dl_
     void *pxn, *pzb, *phb;       // bf16 [maxPrefill][dim | qDim | ff]
     float *pAttnPartial;         // [maxPrefill][nHeads][hd+2]
     unsigned int *pAttnCounters; // [maxPrefill][nHeads]
+    int *pTargets;               // [maxPrefill] score targets (global ids, -1 = none)
+    float *pLogprob, *pTopLogprob;   // [maxPrefill] score results
+    int *pTopId;                 // [maxPrefill]
     // fused arg-max scratch
     float *argVal;               // [256]
     int *argIdx;                 // [256]
@@ -74,6 +77,7 @@ struct Engine {
     // device sampler state (sampler.cu)
     unsigned long long *rngState = nullptr;
     float *probScratch = nullptr;
+    float *scoreLogits = nullptr;      // [scoreMaxTokens][vocab] logits of a scored chunk (first dl_engine_score call; in `owned`)
     unsigned int *gatherEpoch = nullptr, *gatherBlockCounter = nullptr;
     float **gatherUcDev = nullptr;
     unsigned int **flagUcDev = nullptr;
@@ -314,8 +318,9 @@ static int engineForward(Engine &e, int nb, int logitsMode, bool greedyAdvance, 
     return 0;
 }
 
-// Prompt chunk of T <= maxPrefill tokens on the tensor-core path. Logits (optional) are produced for the last token.
-static int enginePrefill(Engine &e, uint32_t T, uint32_t p0, int wantLogits, cudaStream_t stream) {
+// The layers of a prompt chunk of T <= maxPrefill tokens on the tensor-core path: writes the chunk's KV rows and leaves the final
+// residual stream of every token in px.
+static int prefillLayers(Engine &e, uint32_t T, uint32_t p0, cudaStream_t stream) {
     const EngineConfig &c = e.cfg;
     const GlobalPtrs &g = e.g;
     const Buffers &b = e.b;
@@ -387,6 +392,15 @@ static int enginePrefill(Engine &e, uint32_t T, uint32_t p0, int wantLogits, cud
         } else if (tp) { arP.parity = 1; DL_TRY(gemmQ40TcAr(L.w2Qs, L.w2Sc, c.dim, c.ffDim, b.phb, c.ffDim, T, b.px, c.dim, c.numSms, stream, arP)); }
         else DL_TRY(gemmQ40Tc(GEPI_RESIDUAL_, L.w2Qs, L.w2Sc, c.dim, c.ffDim, b.phb, c.ffDim, T, b.px, c.dim, c.numSms, stream, pdl));
     }
+    return 0;
+}
+
+// Prompt chunk of T <= maxPrefill tokens on the tensor-core path. Logits (optional) are produced for the last token.
+static int enginePrefill(Engine &e, uint32_t T, uint32_t p0, int wantLogits, cudaStream_t stream) {
+    const EngineConfig &c = e.cfg;
+    const GlobalPtrs &g = e.g;
+    const Buffers &b = e.b;
+    DL_TRY(prefillLayers(e, T, p0, stream));
     if (wantLogits) {
         GemvArgs a{};
         a.qs = (const uint32_t *)g.wclsQs; a.scales = (const __half *)g.wclsSc; a.d = c.vocab; a.n = c.dim;
@@ -395,6 +409,45 @@ static int enginePrefill(Engine &e, uint32_t T, uint32_t p0, int wantLogits, cud
         DL_TRY(gemvSel(e, PRO_RMSNORM_, EPI_STORE_, 1, a, c.numSms, stream, false));
     }
     return 0;
+}
+
+// Tokens per dl_engine_score call: the chunk limit of the prefill chain, and under tensor parallelism also the rows whose score
+// records fit into one parity of the decode all-reduce slots (maxBatch * dim words per source rank; maxBatch is 1 for MoE models).
+static uint32_t scoreMaxTokens(const EngineConfig &c) {
+    if (c.nRanks <= 1) return c.maxPrefill;
+    return std::min(c.maxPrefill, c.maxBatch * c.dim / kScoreWordsPerRow);
+}
+
+// Prompt chunk on the tensor-core path, then the logits of all T tokens and their scores against the targets staged in pTargets.
+static int engineScore(Engine &e, uint32_t T, uint32_t p0, cudaStream_t stream) {
+    const EngineConfig &c = e.cfg;
+    const Buffers &b = e.b;
+    const bool pdl = c.usePdl != 0;
+    const uint32_t maxT = scoreMaxTokens(c);
+    if (T < 1 || T > maxT) return -11;
+    if (c.wType != 0) return -35;
+    if (c.nRanks > 1 && !e.tp) return -37;
+    if (!e.scoreLogits) {   // [maxScore][vocab] f32, allocated on the first call so that engines that never score keep their footprint
+        void *p = nullptr;
+        DL_CUDA_CHECK(cudaMalloc(&p, (size_t)maxT * c.vocab * sizeof(float)));
+        e.owned.push_back(p);
+        e.scoreLogits = (float *)p;
+    }
+    DL_TRY(prefillLayers(e, T, p0, stream));
+    DL_TRY(launchRmsNormBf16(b.px, c.dim, e.g.finalNorm, b.pxn, c.dim, c.dim, c.eps, T, stream, pdl));
+    DL_TRY(gemmQ40Tc(GEPI_STORE_F32_, e.g.wclsQs, e.g.wclsSc, c.vocab, c.dim, b.pxn, c.dim, T, e.scoreLogits, c.vocab, c.numSms, stream, pdl));
+    ScoreArgs s{};
+    s.logits = e.scoreLogits; s.T = T; s.vocab = c.vocab; s.ld = c.vocab; s.targets = b.pTargets; s.limit = e.vocabLimit;
+    s.rowOffset = c.rank * c.vocab; s.outLogprob = b.pLogprob; s.outTopId = b.pTopId; s.outTopLogprob = b.pTopLogprob;
+    // The records travel through parity 1 of the decode all-reduce slots. Every use of a slot word is a write by the source rank
+    // followed by a read-and-reset by the owning rank, so a write must not land before the previous use's reset. Rank A writes
+    // rank B's words in this kernel only after its own prefill all-reduces of this chunk, which read words that B wrote after
+    // finishing, in stream order, whatever B ran before (a decode step's W2 / MoE all-reduce on parity 1, or the previous
+    // chunk's score kernel): those resets are done. In the other direction, the next user of parity 1 on A (a decode step's W2
+    // or MoE all-reduce, or the next chunk's score) comes after a parity-0 WO all-reduce or the next chunk's prefill all-reduces,
+    // which need B's contribution, written after B's score kernel and its resets completed.
+    if (e.tp) fillAr(e, s.ar, 1);
+    return launchScoreRows(s, stream, pdl);
 }
 
 // Allocates and zeroes the working buffers and KV caches on the current device, finished before it returns: a forward may
@@ -425,6 +478,8 @@ static bool allocBuffers(Engine &e) {
     b.px = (float *)zeroed(mp * dim * 4); b.pqkv = (float *)zeroed(mp * std::max(qkvDim, dim) * 4);
     b.pxn = zeroed(mp * dim * 2); b.pzb = zeroed(mp * qDim * 2); b.phb = zeroed(mp * ff * 2);
     b.pAttnPartial = (float *)zeroed(mp * heads * (hd + 2) * 4); b.pAttnCounters = (unsigned int *)zeroed(mp * heads * 4);
+    b.pTargets = (int *)zeroed(mp * 4); b.pLogprob = (float *)zeroed(mp * 4); b.pTopId = (int *)zeroed(mp * 4);
+    b.pTopLogprob = (float *)zeroed(mp * 4);
     b.argVal = (float *)zeroed(256 * 4); b.argIdx = (int *)zeroed(256 * 4); b.argCounter = (unsigned int *)zeroed(4 * 4);
     for (uint32_t l = 0; l < c.nLayers; l++) {
         e.kCache.push_back(zeroed((size_t)c.nKvHeads * c.seqLen * hd * 2));
@@ -494,9 +549,12 @@ DL_EXPORT int dl_engine_get_config(void *h, dl::EngineConfig *cfg) {
 DL_EXPORT int dl_engine_buffers(void *h, dl::EngineBuffers *out) {
     const Engine *e = (Engine *)h;
     const dl::Buffers &b = e->b;
-    *out = dl::EngineBuffers{b.tokens, b.pos, b.history, b.logits, b.x, b.pTokens, b.pPos, e->kCache.data(), e->vCache.data()};
+    *out = dl::EngineBuffers{b.tokens, b.pos, b.history, b.logits, b.x, b.pTokens, b.pPos, e->kCache.data(), e->vCache.data(),
+                             b.pTargets, b.pLogprob, b.pTopId, b.pTopLogprob};
     return 0;
 }
+
+DL_EXPORT uint32_t dl_engine_score_max_tokens(void *h) { return dl::scoreMaxTokens(((Engine *)h)->cfg); }
 
 DL_EXPORT size_t dl_engine_arena_bytes(const dl::EngineConfig *cfg) { return dl::arenaLayout(dl::applyLimits(*cfg)).bytes; }
 
@@ -703,6 +761,10 @@ DL_EXPORT int dl_engine_forward_part(void *h, int nb, uint32_t layer, int part, 
 
 DL_EXPORT int dl_engine_prefill(void *h, uint32_t T, uint32_t p0, int wantLogits, cudaStream_t stream) {
     return dl::enginePrefill(*(Engine *)h, T, p0, wantLogits, stream);
+}
+
+DL_EXPORT int dl_engine_score(void *h, uint32_t T, uint32_t p0, cudaStream_t stream) {
+    return dl::engineScore(*(Engine *)h, T, p0, stream);
 }
 
 // Captures one greedy decode step (forward of 1 token + argmax + position advance) into a graph.

@@ -50,6 +50,10 @@ struct EngineBuffers {
     float *x;                    // [maxBatch][dim] residual stream
     int *pTokens, *pPos;         // [maxPrefill] tokens and positions of a prefill chunk
     void *const *kCache, *const *vCache;   // [nLayers] (host arrays) bf16 [nKvHeads][seqLen][hd]
+    int *pTargets;               // [maxPrefill] dl_engine_score: target of each row (global id, -1 = none)
+    float *pLogprob;             // [maxPrefill] dl_engine_score results: log P(target), NaN without a target
+    int *pTopId;                 //              top-1 id (ids >= the vocabulary limit excluded, lowest index on ties)
+    float *pTopLogprob;          //              its log-probability
 };
 
 struct CommPtrs {   // mirrored by ctypes
@@ -80,6 +84,11 @@ int dl_engine_set_trace_all(void *h, int allCtas);
 int dl_engine_forward(void *h, int nb, int logitsMode, int greedyAdvance, cudaStream_t stream);
 int dl_engine_forward_part(void *h, int nb, uint32_t layer, int part, float *ybuf, cudaStream_t stream);
 int dl_engine_prefill(void *h, uint32_t T, uint32_t p0, int wantLogits, cudaStream_t stream);   // T tokens staged in pTokens/pPos at positions p0 .. p0 + T - 1
+// Scores T tokens staged in pTokens/pPos/pTargets at positions p0 .. p0 + T - 1: the prefill chain (same KV rows as dl_engine_prefill),
+// the logits of every token, then log-probabilities over the whole vocabulary into pLogprob/pTopId/pTopLogprob. Every rank of a
+// tensor-parallel job gets bit-identical results. T <= dl_engine_score_max_tokens; -35 for dense weight files.
+int dl_engine_score(void *h, uint32_t T, uint32_t p0, cudaStream_t stream);
+uint32_t dl_engine_score_max_tokens(void *h);
 int dl_engine_capture_decode(void *h);
 int dl_engine_decode_graph(void *h, int nSteps, cudaStream_t stream);
 // symmetric peer-memory arena (csrc/cuda/comm_vmm.cu): create (local, binds the bootstrap socket) -> [job-wide barrier] -> connect

@@ -238,6 +238,21 @@ inline cudaError_t launchPdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, si
     return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
+// Prompt scoring (score.cu): log-probability of each row's target, top-1 id and its log-probability, from f32 logits rows.
+constexpr uint32_t kScoreWordsPerRow = 4;   // LL words per row and source rank in the tensor-parallel record exchange
+struct ScoreArgs {
+    const float *logits;          // [T][ld], this rank's vocabulary slice
+    uint32_t T, vocab, ld;        // rows, local vocabulary entries per row, row stride
+    const int *targets;           // [T] global target ids, -1 = none
+    uint32_t limit;               // global ids >= limit never win the top-1 (0 = no limit)
+    uint32_t rowOffset;           // global id of local entry 0 (rank * vocab)
+    float *outLogprob;            // [T] (NaN where the target is -1)
+    int *outTopId;                // [T] global id
+    float *outTopLogprob;         // [T]
+    ArArgs ar;                    // ar.nRanks > 1: records exchanged over the peer arena, slot words [t * kScoreWordsPerRow, +4)
+};
+int launchScoreRows(const ScoreArgs &a, cudaStream_t stream, bool pdl);
+
 int launchArResidual(float *x, const float *partial, uint32_t dim, uint32_t T, const ArArgs &ar, cudaStream_t stream, bool pdl = false);   // x += all-reduce(partial)
 int launchRmsNormBf16(const float *x, uint32_t xStride, const float *w, void *y, uint32_t yStride, uint32_t n, float eps, uint32_t T,
                       cudaStream_t stream, bool pdl = false);

@@ -66,6 +66,14 @@ class InferenceSession:
             self.engine.prefill(tokens, self.pos, want_logits=False)
             self.pos += len(tokens)
 
+    def score(self, tokens: Sequence[int]):
+        """Evaluates tokens at positions pos..pos+n-1 and returns their scores (runtime.engine.ScoreResult: log P(tokens[i+1] |
+        tokens[..i]), top-1 ids and log-probabilities). Advances pos by n-1, like prefill(tokens[:-1]): feeding tokens[-1] to
+        next_token continues the sequence."""
+        res = self.engine.score(tokens, self.pos)
+        self.pos += len(tokens) - 1
+        return res
+
     def forward_logits(self, token: int) -> torch.Tensor:
         lg = self.engine.step(token, self.pos)
         self.pos += 1

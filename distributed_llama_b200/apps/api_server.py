@@ -1,6 +1,7 @@
 """`dllama-api`: OpenAI-style HTTP server (reference src/dllama-api.cpp:43-632, src/api-types.hpp).
 
-Routes: POST /v1/chat/completions (JSON or SSE-chunked stream), GET /v1/models, OPTIONS * (CORS pre-flight), else 404.
+Routes: POST /v1/chat/completions (JSON or SSE-chunked stream), POST /v1/completions (prompt log-probabilities and plain
+completions, JSON only), GET /v1/models, OPTIONS * (CORS pre-flight), else 404.
 Single request at a time over one global KV sequence, with the reference's NaiveCache prefix reuse: if the new message
 history extends the cached one, generation restarts from the cached end position instead of 0.
 Deliberate fixes over the reference (SURVEY A.2): request `temperature`/`top_p` are applied, `finish_reason` is "stop"
@@ -100,6 +101,12 @@ class HttpRequest:
         self._send(b"HTTP/1.1 200 OK\r\nAccess-Control-Allow-Origin: *\r\nContent-Type: application/json; charset=utf-8\r\n"
                    b"Connection: close\r\nContent-Length: " + str(len(body)).encode() + b"\r\n\r\n" + body)
 
+    def write_error(self, status: int, message: str):
+        body = json.dumps({"error": {"message": message, "type": "invalid_request_error"}}).encode("utf-8")
+        reason = {400: "Bad Request"}.get(status, "Error")
+        self._send(f"HTTP/1.1 {status} {reason}\r\n".encode() + b"Access-Control-Allow-Origin: *\r\nContent-Type: application/json; charset=utf-8\r\n"
+                   b"Connection: close\r\nContent-Length: " + str(len(body)).encode() + b"\r\n\r\n" + body)
+
     def write_stream_start(self):
         self._send(b"HTTP/1.1 200 OK\r\nAccess-Control-Allow-Origin: *\r\nContent-Type: text/event-stream; charset=utf-8\r\n"
                    b"Connection: close\r\nTransfer-Encoding: chunked\r\n\r\n")
@@ -196,6 +203,73 @@ class ApiServer:
                 "choices": [{"index": 0, "message": {"role": "assistant", "content": buffer}, "finish_reason": "stop"}]}))
         print("🔶")
 
+    def text_completion(self, req: HttpRequest):
+        """POST /v1/completions, the OpenAI legacy completions contract that evaluation harnesses use for log-likelihoods. The
+        prompt is tokenized with BOS and no chat template. With `echo` and `logprobs`, the prompt is scored on the device
+        (InferenceSession.score), which is also its prefill; generated tokens come from the decode loop, and with `logprobs` one
+        score pass over the last prompt token and the completion gives their log-probabilities afterwards. `tokens[i]` is the text
+        the tokenizer's decoder emits for token i, and `text_offset[i]` its character offset in `text`."""
+        ctx = self.ctx
+        tok, inf, h, smp = ctx.tokenizer, ctx.inference, ctx.header, ctx.sampler
+        body = req.json if isinstance(req.json, dict) else {}
+        prompt, logprobs, max_tokens = body.get("prompt"), body.get("logprobs"), body.get("max_tokens", 16)
+        if body.get("stream"):
+            return req.write_error(400, "stream is not supported on /v1/completions")
+        if not isinstance(prompt, str):
+            return req.write_error(400, "prompt must be a string")
+        if logprobs is not None and (type(logprobs) is not int or not 0 <= logprobs <= 1):
+            return req.write_error(400, "logprobs must be null, 0 or 1")
+        if type(max_tokens) is not int or max_tokens < 0:
+            return req.write_error(400, "max_tokens must be a non-negative integer")
+        tokens = list(tok.encode(prompt, True, True))
+        n = len(tokens)
+        if n > h.seq_len:
+            return req.write_error(400, f"the prompt has {n} tokens, more than the context length ({h.seq_len})")
+        echo = bool(body.get("echo", False))
+        smp.set_temperature(float(body.get("temperature", ctx.args.temperature)))
+        smp.set_topp(float(body.get("top_p", ctx.args.topp)))
+        if "seed" in body:
+            smp.set_seed(int(body["seed"]))
+        self.cache.clear()   # this request overwrites the KV rows the chat cache points at
+        prompt_scores = None
+        if echo and logprobs is not None:
+            prompt_scores = inf.score(tokens, 0)
+        else:
+            inf.prefill(tokens[:-1], 0)
+        pos, token, generated, finish = n - 1, tokens[-1], [], "length"
+        while len(generated) < max_tokens and pos < h.seq_len:
+            token = inf.next_token(token, pos, smp)
+            pos += 1
+            if tok.is_eos(token):
+                finish = "stop"
+                break
+            generated.append(token)
+        tok.reset_decoder()
+        ids = (tokens if echo else []) + generated
+        strs = [tok.decode(t).decode("utf-8", errors="replace") for t in ids]
+        choice = {"index": 0, "text": "".join(strs), "logprobs": None, "finish_reason": finish}
+        if logprobs is not None:
+            def top(i, lp):
+                return {tok.piece(i).decode("utf-8", errors="replace"): lp} if logprobs else {}
+            token_lp, top_lp = [], []
+            if echo:
+                token_lp = [None] + prompt_scores.logprobs.tolist()
+                top_lp = [None] + [top(i, lp) for i, lp in zip(prompt_scores.top_ids.tolist()[:n - 1], prompt_scores.top_logprobs.tolist())]
+            if generated:
+                s = inf.score([tokens[-1]] + generated[:-1], n - 1, next_token=generated[-1])
+                token_lp += s.logprobs.tolist()
+                top_lp += [top(i, lp) for i, lp in zip(s.top_ids.tolist(), s.top_logprobs.tolist())]
+            offsets, off = [], 0
+            for s_ in strs:
+                offsets.append(off)
+                off += len(s_)
+            choice["logprobs"] = {"tokens": strs, "token_logprobs": token_lp, "top_logprobs": top_lp, "text_offset": offsets}
+        n_completion = len(generated)
+        req.write_json(json.dumps({
+            "id": "cmpl-t0", "object": "text_completion", "created": int(time.time()), "model": "Distributed Model",
+            "usage": {"completion_tokens": n_completion, "prompt_tokens": n, "total_tokens": n + n_completion},
+            "choices": [choice]}))
+
     def models(self, req: HttpRequest):
         name = self.ctx.args.model.replace("\\", "/").split("/")[-1]
         req.write_json(json.dumps({"object": "list", "data": [{"id": name, "object": "model", "created": 0, "owned_by": "user"}]}))
@@ -220,6 +294,8 @@ def serve(ctx: AppContext, max_requests: int = 0) -> None:
                 req.write_cors()
             elif req.method == "POST" and req.path == "/v1/chat/completions":
                 api.complete(req)
+            elif req.method == "POST" and req.path == "/v1/completions":
+                api.text_completion(req)
             elif req.method == "GET" and req.path == "/v1/models":
                 api.models(req)
             else:

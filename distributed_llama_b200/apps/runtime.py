@@ -20,7 +20,7 @@ from .. import host
 from ..api import InferenceSession
 from .args import AppArgs
 
-OP_STOP, OP_PREFILL, OP_STEP_LOGITS, OP_STEP_GREEDY, OP_DECODE_N, OP_STEP_SAMPLE, OP_SEED = 0, 1, 2, 3, 4, 5, 6
+OP_STOP, OP_PREFILL, OP_STEP_LOGITS, OP_STEP_GREEDY, OP_DECODE_N, OP_STEP_SAMPLE, OP_SEED, OP_SCORE = 0, 1, 2, 3, 4, 5, 6, 7
 
 
 def world():
@@ -100,6 +100,21 @@ class RootInference:
         if tokens:
             self._send(OP_PREFILL, pos, tokens)
             self.eng.prefill(tokens, pos, want_logits=False)
+
+    def score(self, tokens: Sequence[int], pos: int, next_token: Optional[int] = None):
+        """Scores tokens at positions pos.. (Engine.score). One OP_SCORE packet per piece that fits a control packet: the piece,
+        then the token that follows it (-1: none), so the pieces' scores join up exactly."""
+        from ..parallel.control import MAX_TOKENS
+        from ..runtime.engine import ScoreResult
+        tokens = list(tokens)
+        step = MAX_TOKENS - 1
+        parts = []
+        for i in range(0, len(tokens), step):
+            piece = tokens[i:i + step]
+            nxt = tokens[i + step] if i + step < len(tokens) else next_token
+            self._send(OP_SCORE, pos + i, piece + [-1 if nxt is None else nxt])
+            parts.append(self.eng.score(piece, pos + i, next_token=nxt))
+        return ScoreResult.cat(parts)
 
     def forward_logits(self, token: int, pos: int) -> torch.Tensor:
         self._send(OP_STEP_LOGITS, pos, [token])
@@ -195,6 +210,8 @@ def worker_loop(sess: InferenceSession, comm, chan=None) -> None:
             eng.run_decode_step()
         elif op == OP_DECODE_N:
             eng.decode_greedy(toks[0], pos, toks[1])
+        elif op == OP_SCORE:
+            eng.score(toks[:-1], pos, next_token=None if toks[-1] < 0 else toks[-1])
         elif op == OP_SEED:
             eng.seed_sampler(toks[0] | (toks[1] << 31) | (toks[2] << 62))
         elif op == OP_STEP_SAMPLE:

@@ -34,7 +34,8 @@ class GlobalPtrs(C.Structure):
 
 class EngineBuffers(C.Structure):
     _fields_ = [(n, vp) for n in ("tokens", "pos", "history", "logits", "x", "pTokens", "pPos")] + \
-               [("kCache", C.POINTER(vp)), ("vCache", C.POINTER(vp))]
+               [("kCache", C.POINTER(vp)), ("vCache", C.POINTER(vp))] + \
+               [(n, vp) for n in ("pTargets", "pLogprob", "pTopId", "pTopLogprob")]
 
 
 class CommPtrs(C.Structure):
@@ -136,6 +137,12 @@ def lib() -> C.CDLL:
     L.dl_engine_forward_part.restype = i32
     L.dl_engine_prefill.argtypes = [vp, u32, u32, i32, vp]
     L.dl_engine_prefill.restype = i32
+    L.dl_engine_score.argtypes = [vp, u32, u32, vp]
+    L.dl_engine_score.restype = i32
+    L.dl_engine_score_max_tokens.argtypes = [vp]
+    L.dl_engine_score_max_tokens.restype = u32
+    L.dl_score_rows.argtypes = [vp, u32, u32, u32, vp, u32, vp, vp, vp, vp]
+    L.dl_score_rows.restype = i32
     L.dl_engine_capture_decode.argtypes = [vp]
     L.dl_engine_capture_decode.restype = i32
     L.dl_engine_decode_graph.argtypes = [vp, i32, vp]
@@ -151,6 +158,7 @@ _ERRORS = {
     -32: "mixture-of-experts down-projection shape not covered by the TMA GEMV (per-rank expert ffDim must be a multiple of 128: use moe_mode=ep)",
     -33: "arg-max under tensor parallelism needs the fused logits kernel",
     -36: "mixture-of-experts prefill shape not covered (dim, ffDim multiples of 256, chunk <= 256 tokens)",
+    -37: "scoring under tensor parallelism needs the peer arena (fused collectives)",
 }
 
 

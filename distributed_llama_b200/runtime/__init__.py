@@ -1,1 +1,1 @@
-from .engine import Engine
+from .engine import Engine, ScoreResult

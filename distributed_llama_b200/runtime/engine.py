@@ -9,6 +9,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+from dataclasses import dataclass
 from typing import List, Optional, Sequence
 
 import numpy as np
@@ -16,6 +17,20 @@ import torch
 
 from ..models.loader import DeviceWeights
 from ..ops import cuda_lib as cl
+
+
+@dataclass
+class ScoreResult:
+    """Scores of a token sequence t[0..n): `logprobs[i]` = log P(t[i+1] | t[..i]) (length n-1, or n when the following token was
+    given), `top_ids[i]` / `top_logprobs[i]` = the most likely token after t[..i] and its log-probability (length n). CPU tensors."""
+    logprobs: torch.Tensor       # float32
+    top_ids: torch.Tensor        # int32
+    top_logprobs: torch.Tensor   # float32
+
+    @staticmethod
+    def cat(parts: Sequence["ScoreResult"]) -> "ScoreResult":
+        return ScoreResult(torch.cat([p.logprobs for p in parts]), torch.cat([p.top_ids for p in parts]),
+                           torch.cat([p.top_logprobs for p in parts]))
 
 
 def _p(t: Optional[torch.Tensor]):
@@ -91,6 +106,8 @@ class Engine:
         self.tokens, self.pos, self.history = view(b.tokens, (mb,)), view(b.pos, (mb,)), view(b.history, (self.seq_len + 1,))
         self.logits, self.x = view(b.logits, (mb, w.vocab), torch.float32), view(b.x, (mb, h.dim), torch.float32)
         self.p_tokens, self.p_pos = view(b.pTokens, (mp,)), view(b.pPos, (mp,))
+        self.p_targets, self.p_top_id = view(b.pTargets, (mp,)), view(b.pTopId, (mp,))
+        self.p_logprob, self.p_top_logprob = view(b.pLogprob, (mp,), torch.float32), view(b.pTopLogprob, (mp,), torch.float32)
         kv = (w.n_kv_heads, self.seq_len, h.head_dim)
         self.k_cache = [view(b.kCache[l], kv, torch.bfloat16) for l in range(h.n_layers)]
         self.v_cache = [view(b.vCache[l], kv, torch.bfloat16) for l in range(h.n_layers)]
@@ -113,6 +130,7 @@ class Engine:
         if h.n_experts == 0 and not self.dense and not self._parts and os.environ.get("DL_NO_MEGA") is None:
             self.enable_mega(True)     # persistent decode kernel by default; the engine falls back per call if a shape is unsupported
         self.tc_min_tokens = 9          # shorter chunks stay on the GEMV path
+        self._vocab_limit = 0
         self._graph_ready = False
         self._stage_tok = torch.zeros(mb, dtype=torch.int32).pin_memory()
         self._stage_pos = torch.zeros(mb, dtype=torch.int32).pin_memory()
@@ -121,6 +139,7 @@ class Engine:
         """Greedy arg-max on the device never returns ids >= limit (the tokenizer's vocabulary size: embeddings may be padded
         beyond it, reference src/app.cpp:243-246 builds its sampler on the tokenizer size too)."""
         cl.check(self._lib.dl_engine_set_vocab_limit(self._h, int(limit)), "engine_set_vocab_limit")
+        self._vocab_limit = int(limit)
         self._graph_ready = False
 
     # -- device-side sampling --
@@ -217,13 +236,7 @@ class Engine:
         tokens = list(tokens)
         if start_pos + len(tokens) > self.seq_len:
             raise ValueError("position beyond the context length")
-        hdr = self.w.header
-        tp = self.comm is not None and self.comm.world_size > 1
-        # tensor parallel: the fused GEMM + all-reduce kernel needs 256-wide K slices on every rank
-        tp_ok = (not tp) or ((self.w.n_heads * hdr.head_dim) % 256 == 0 and self.w.ff_dim % 256 == 0 and hdr.dim % 256 == 0)
-        # mixture of experts: the grouped tensor-core GEMMs need 256-wide K on both expert matrices
-        moe_ok = hdr.n_experts == 0 or (hdr.dim % 256 == 0 and self.w.ff_dim % 256 == 0 and os.environ.get("DL_NO_MOE_PREFILL") is None)
-        tc_path = tp_ok and moe_ok and self.use_tc_prefill
+        tc_path = self._tc_prefill_ok()
         i = 0
         while i < len(tokens):
             rem = len(tokens) - i
@@ -241,6 +254,63 @@ class Engine:
                 self.forward_batch(tokens[i:i + n], start_pos + i, logits_mode=1 if (last and want_logits) else 0)
             i += n
         return self._full_logits(self.logits[0]) if want_logits else None
+
+    def _tc_prefill_ok(self) -> bool:
+        """Whether prompt chunks can take the tensor-core path (dl_engine_prefill / dl_engine_score) on this configuration."""
+        hdr = self.w.header
+        tp = self.comm is not None and self.comm.world_size > 1
+        # tensor parallel: the fused GEMM + all-reduce kernel needs 256-wide K slices on every rank
+        tp_ok = (not tp) or ((self.w.n_heads * hdr.head_dim) % 256 == 0 and self.w.ff_dim % 256 == 0 and hdr.dim % 256 == 0)
+        # mixture of experts: the grouped tensor-core GEMMs need 256-wide K on both expert matrices
+        moe_ok = hdr.n_experts == 0 or (hdr.dim % 256 == 0 and self.w.ff_dim % 256 == 0 and os.environ.get("DL_NO_MOE_PREFILL") is None)
+        return tp_ok and moe_ok and self.use_tc_prefill
+
+    @property
+    def score_max_tokens(self) -> int:
+        """Tokens per dl_engine_score call (prefill chunk limit; under tensor parallelism also the record-exchange capacity)."""
+        return int(self._lib.dl_engine_score_max_tokens(self._h))
+
+    def score(self, tokens: Sequence[int], start_pos: int = 0, next_token: Optional[int] = None) -> ScoreResult:
+        """Evaluates tokens at positions start_pos.. (writing the same KV rows as `prefill`) and scores every next token on the
+        device: see ScoreResult. `next_token`, the token that follows `tokens`, adds its log-probability as a last entry.
+        Tensor-core path: chunks of `score_max_tokens`, logits of all tokens by one GEMM, log-softmax by csrc/cuda/score.cu; the
+        target of a chunk's last row is the first token of the next chunk. Where that path does not run (dense weight files, the
+        library-collective mode, shapes the tensor-core prefill does not cover) the logits come from the GEMV batches and are
+        normalised with torch.log_softmax on the device. Under tensor parallelism every rank must make the same call."""
+        tokens = [int(t) for t in tokens]
+        n = len(tokens)
+        if n == 0:
+            raise ValueError("nothing to score")
+        if start_pos + n > self.seq_len:
+            raise ValueError("position beyond the context length")
+        targets = tokens[1:] + [-1 if next_token is None else int(next_token)]
+        lp, ids, top = [], [], []
+        if self._tc_prefill_ok():
+            cap = self.score_max_tokens
+            for i in range(0, n, cap):
+                m = min(cap, n - i)
+                self.p_tokens[:m].copy_(torch.tensor(tokens[i:i + m], dtype=torch.int32))
+                self.p_pos[:m].copy_(torch.arange(start_pos + i, start_pos + i + m, dtype=torch.int32))
+                self.p_targets[:m].copy_(torch.tensor(targets[i:i + m], dtype=torch.int32))
+                cl.check(self._lib.dl_engine_score(self._h, m, start_pos + i, cl.stream_ptr()), "engine_score")
+                lp.append(self.p_logprob[:m].clone()); ids.append(self.p_top_id[:m].clone()); top.append(self.p_top_logprob[:m].clone())
+        else:
+            limit = self._vocab_limit
+            i = 0
+            while i < n:
+                nb = 1
+                while nb * 2 <= min(n - i, self.max_batch):
+                    nb *= 2
+                lsm = torch.log_softmax(self.logits_all(tokens[i:i + nb], start_pos + i).float(), dim=-1)
+                tv = lsm[:, :limit] if 0 < limit < lsm.shape[1] else lsm
+                best = tv.argmax(dim=-1)                       # first maximal index: the lowest id wins ties
+                tg = torch.tensor(targets[i:i + nb], dtype=torch.int64, device=lsm.device)
+                got = lsm.gather(1, tg.clamp(min=0)[:, None])[:, 0]
+                lp.append(torch.where(tg >= 0, got, torch.full_like(got, float("nan"))))
+                ids.append(best.to(torch.int32)); top.append(lsm.gather(1, best[:, None])[:, 0])
+                i += nb
+        n_lp = n if next_token is not None else n - 1
+        return ScoreResult(torch.cat(lp)[:n_lp].cpu(), torch.cat(ids).cpu(), torch.cat(top).cpu())
 
     def step(self, token: int, pos: int) -> torch.Tensor:
         """Forward of one token; returns the full-vocabulary logits row (gathered over ranks under tensor parallelism)."""

@@ -1,5 +1,5 @@
 """Workload for compute-sanitizer (tools/sanitize.sh): tiny synthetic models through every kernel family — tcgen05 prefill,
-persistent decode kernel, multi-kernel PDL decode path, MoE router + routed GEMVs, dense f32 weights."""
+persistent decode kernel, multi-kernel PDL decode path, MoE router + routed GEMVs, dense f32 weights, prompt scoring."""
 import os
 import sys
 import tempfile
@@ -32,4 +32,8 @@ with tempfile.TemporaryDirectory() as d:
             eng.step(toks[-1], len(prompt) + 5)
             torch.cuda.synchronize()
             print(spec, "mega" if eng.mega else "multi-kernel", toks)
+        # prompt scoring: prefill chain + logits GEMM + score kernel in chunks of 64 (dense files: the GEMV fallback)
+        res = Engine(load_device_weights(mf), max_prefill=64).score([(3 * i + 1) % 500 + 1 for i in range(150)], 0)
+        torch.cuda.synchronize()
+        print(spec, "score", res.top_ids[:6].tolist())
 print("SANITIZE_TARGET_DONE")
